@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA engine
     python bench.py --impl reference --gpus N --steps K --warmup W   # reference CPU path (oracle port)
     torchrun ... bench.py --gpus N ...                        # one rank per GPU, filters sharded by index
+    python bench.py ... --dump-outputs DIR                    # also write the state the timed steps computed
 
 Workload (BASELINE.json config 4 at one GPU, SURVEY.md section 8(d) "C4"): 1,048,576
 PoseUKF instances per GPU, Monte-Carlo initial states, one step = predictionStep(dt = 1 ms)
@@ -182,6 +183,26 @@ def parity_sample(applied, indices, mu_gpu, sg_gpu, pool: int):
             "tolerance": 1e-9}
 
 
+DUMP_FILTERS = 32768  # mu + sigma of this many filters: 41 MB of float64
+
+
+def dump_outputs(out_dir, f, dev):
+    """--dump-outputs: the state estimates (ukfb_get_state) of a fixed sample of DUMP_FILTERS filters (seeded, in index
+    order; every filter when there are fewer) as DIR/mu.npy (S x 13) and DIR/sigma.npy (S x 12 x 12), float64.  The
+    inputs depend on the arguments only, so two builds of the engine can be compared output for output."""
+    import torch
+
+    B = f.B
+    idx = np.arange(B) if B <= DUMP_FILTERS else np.sort(np.random.default_rng(0).choice(B, DUMP_FILTERS, replace=False))
+    d_mu = torch.empty((B, f.MU), dtype=torch.float64, device=dev)
+    d_sg = torch.empty((B, f.n, f.n), dtype=torch.float64, device=dev)
+    f.get_state_dev(d_mu, d_sg)
+    d_idx = torch.from_numpy(idx).to(dev)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "mu.npy"), d_mu[d_idx].cpu().numpy())
+    np.save(os.path.join(out_dir, "sigma.npy"), d_sg[d_idx].cpu().numpy())
+
+
 def run_reference(args, rank, world):
     """--impl reference: the reference's CPU path (cpu_arm: oracle/_ref, else the oracle port), OpenMP over filters on
     all host cores.  Rank 0 only."""
@@ -244,7 +265,11 @@ def main():
     ap.add_argument("--no-literal", action="store_true", help="skip the secondary measurement of the literal kernel")
     ap.add_argument("--no-orientation", action="store_true", help="skip the secondary OrientationUKF (C2) figure")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling leg (1 Mi filters in total) at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the state after the last timed step (a fixed sample of "
+                                                          "rank 0's filters) to DIR/mu.npy and DIR/sigma.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
@@ -319,6 +344,8 @@ def main():
     launches = f.launch_count() - launches0
     hist = f.get_mean_iter_hist()
     n_flag, bits = f.status_summary()
+    if args.dump_outputs and rank == 0:  # before the end-to-end legs below take further steps on f
+        dump_outputs(args.dump_outputs, f, dev)
 
     # ---- end to end through the host-pointer C ABI ----------------------------------------------
     # Every step: H2D of that step's measurements from pinned host memory, the fused kernel, D2H of the estimates into
