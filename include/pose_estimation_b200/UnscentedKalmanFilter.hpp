@@ -88,6 +88,34 @@ public:
         return getCurrentState(&state, nullptr);
     }
 
+    /* The reference's single-filter calls for filter `index` of this object (a global index, also across devices): what a
+     * caller owning N reference objects does to the one it needs, here without touching the others.  initializeFilter
+     * resets that filter's time latch (:43) and leaves its status word alone. */
+    void initializeFilter(int64_t index, const State& initial_state, const Covariance& state_cov)
+    {
+        check(ukfb_initialize_indexed(h, 1, &index, initial_state.v, state_cov.v));
+    }
+    bool getCurrentState(int64_t index, State& state, Covariance& state_cov) const
+    {
+        return getCurrentStates(1, &index, &state, &state_cov);
+    }
+    bool getCurrentState(int64_t index, State& state) const { return getCurrentStates(1, &index, &state, nullptr); }
+    /* the same for n filters idx[0..n) at once: entry k of the arrays belongs to filter idx[k] (unique for initialize) */
+    void initializeFilters(int64_t n, const int64_t* idx, const State* initial_states, const Covariance* state_covs)
+    {
+        check(ukfb_initialize_indexed(h, n, idx, n ? initial_states->v : nullptr, n ? state_covs->v : nullptr));
+    }
+    bool getCurrentStates(int64_t n, const int64_t* idx, State* states, Covariance* state_covs) const
+    {
+        const int rc = ukfb_get_state_indexed(h, n, idx, n ? states->v : nullptr, n && state_covs ? state_covs->v : nullptr);
+        if (rc == UKFB_ERR_NOT_INITIALIZED) return false;
+        check(rc);
+        return true;
+    }
+    /* the filters whose condition the last exception reported (ascending), for getting them back with
+     * initializeFilter(index, ...); empty after a call that threw nothing */
+    const std::vector<int64_t>& lastFailedFilters() const { return failed; }
+
     /* :83-100; sample_time in microseconds (base::Time::microseconds) */
     void predictionStepFromSampleTime(int64_t sample_time_us)
     {
@@ -154,8 +182,17 @@ protected:
     {
         int64_t n = 0;
         uint32_t bits = 0;
+        failed.clear();
         check(ukfb_status_summary(h, &n, &bits));
         if (!bits) return;
+        const uint32_t thrown = UKFB_STATUS_NEG_DT | UKFB_STATUS_DT_TOO_LARGE | UKFB_STATUS_NONFINITE_MEAS | UKFB_STATUS_NOT_SPD |
+                                UKFB_STATUS_MEAN_NO_CONVERGE;
+        if (bits & thrown) { /* which filters: before the status words are cleared */
+            int64_t count = 0;
+            check(ukfb_find_status(h, thrown, 0, nullptr, &count));
+            failed.resize(size_t(count));
+            check(ukfb_find_status(h, thrown, count, failed.data(), &count));
+        }
         check(ukfb_clear_status(h));
         if (bits & UKFB_STATUS_NEG_DT) throw std::runtime_error("Delta time is negative!");                               /* :112 */
         if (bits & UKFB_STATUS_DT_TOO_LARGE) throw std::runtime_error("Delta time is greater then the allowed maximum!"); /* :121 */
@@ -182,6 +219,7 @@ protected:
 
     ukfb_handle* h;
     int64_t batch_size;
+    std::vector<int64_t> failed; /* lastFailedFilters() */
 };
 
 }  // namespace pose_estimation_b200

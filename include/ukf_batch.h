@@ -307,6 +307,39 @@ int ukfb_status_summary(ukfb_handle* h, int64_t* n_flagged, uint32_t* any_bits);
 int ukfb_get_mean_iter_hist(ukfb_handle* h, uint64_t hist[8]);
 int ukfb_clear_mean_iter_hist(ukfb_handle* h);
 
+/* ---- per-filter access ------------------------------------------------------------------------------------------ */
+/* A caller of the reference owns N filter objects and calls initializeFilter (UnscentedKalmanFilter.hpp:40-44) or
+ * getCurrentState (:51-75) on the ONE it needs; these calls do that for the filters idx[0..n) of a batch and touch
+ * nothing else (a filter whose status shows UKFB_STATUS_NOT_SPD fails every later factorisation: re-initialising it,
+ * then clearing its status, is how it comes back without disturbing the others).
+ *   - idx: n int64 GLOBAL filter indices (also on a sharded handle), in any order; row k of every data array belongs to
+ *     filter idx[k].  n = 0 is a no-op returning UKFB_OK (null pointers allowed then).
+ *   - host-pointer calls check n < 0, null pointers with n > 0, indices outside [0, B) and (ukfb_initialize_indexed)
+ *     duplicates, and return UKFB_ERR_INVALID before anything is enqueued: a rejected call changes nothing, on any
+ *     shard.  They stage n rows, never B.
+ *   - `_dev` calls take device indices and cannot report per-index errors: they require valid indices (unique for
+ *     initialize).  An index outside [0, B) is skipped (its row is neither read nor written); duplicates in initialize
+ *     leave those filters' records unspecified.  On a sharded parent they return UKFB_ERR_INVALID, as every `_dev` call.
+ *   - all work is plain launches and cudaMemcpyAsync on the handle's stream, in full stream order with the step
+ *     launches before and after (also where those overlap one another tile by tile, see ukfb_overlapped_launch_count).
+ */
+/* getCurrentState of filters idx[0..n): mu n x MU, sigma n x n x n (full symmetric, as ukfb_get_state) or NULL.
+ * Duplicates allowed.  Bit for bit the rows idx[k] of ukfb_get_state. */
+int ukfb_get_state_indexed(ukfb_handle* h, int64_t n, const int64_t* idx, double* mu, double* sigma);
+int ukfb_get_state_indexed_dev(ukfb_handle* h, int64_t n, const int64_t* d_idx, double* d_mu, double* d_sigma);
+/* initializeFilter of filters idx[0..n) only: record replaced (mu, lower triangle of sigma), t_last = 0 (:43).
+ * Q, the stored acceleration / rotation rate, orientation parameters, status words and every other filter are
+ * untouched: status is left alone exactly as ukfb_initialize leaves it, recovery clears it explicitly.  The handle must
+ * already be initialized (the first ukfb_initialize also does the OrientationUKF constructor's defaults):
+ * UKFB_ERR_NOT_INITIALIZED otherwise. */
+int ukfb_initialize_indexed(ukfb_handle* h, int64_t n, const int64_t* idx, const double* mu, const double* sigma);
+int ukfb_initialize_indexed_dev(ukfb_handle* h, int64_t n, const int64_t* d_idx, const double* d_mu, const double* d_sigma);
+/* filters whose status word has any bit of `bits`, ascending; the first min(max_n, count) are written to idx,
+ * *n_found = count (idx may be NULL when max_n = 0: count only) */
+int ukfb_find_status(ukfb_handle* h, uint32_t bits, int64_t max_n, int64_t* idx, int64_t* n_found);
+/* status words of filters idx[0..n) set to 0 (ukfb_clear_status for a subset); duplicates allowed */
+int ukfb_clear_status_indexed(ukfb_handle* h, int64_t n, const int64_t* idx);
+
 /* ---- stream plumbing ------------------------------------------------------- */
 
 int ukfb_synchronize(ukfb_handle* h);

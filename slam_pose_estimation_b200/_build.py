@@ -14,7 +14,9 @@ CSRC = os.path.join(_PKG, "csrc")
 # UKFB_LIB: load another build of the same library (kernel tuning experiments)
 LIB = os.environ.get("UKFB_LIB") or os.path.join(_PKG, "lib", "libukfb.so")
 SOURCES = ["ukf_batch.cu"]
-DEPS = ["ukf_batch.cu", "ukf_device.cuh", "ukf_thread.cuh", "ukf_pose_fast.cuh", "ukf_ori_fast.cuh", "so3.cuh", "simt.cuh", "../../include/ukf_batch.h", "../../include/ukfb_constants.h"]
+DEPS = ["ukf_batch.cu", "ukf_device.cuh", "ukf_thread.cuh", "ukf_pose_fast.cuh", "ukf_ori_fast.cuh", "ukf_index.cuh", "so3.cuh", "simt.cuh", "../../include/ukf_batch.h", "../../include/ukfb_constants.h"]
+# the step kernels' sources: what source_hash() covers (ukf_index.cuh holds per-filter access kernels, no step code)
+STEP_KERNEL_SOURCES = ["simt.cuh", "so3.cuh", "ukf_device.cuh", "ukf_ori_fast.cuh", "ukf_pose_fast.cuh", "ukf_thread.cuh"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
@@ -30,14 +32,15 @@ def nvcc() -> str:
 
 
 def source_hash() -> str:
-    """sha256 (first 16 hex digits) of the KERNEL sources (csrc/*.cuh; the host side of the ABI in ukf_batch.cu does not
-    change what a kernel executes) the library is built from: profiles/traffic.json is stamped with it, so that ncu
-    figures of an older kernel are not reported for a newer one.  Comments and white space do not count."""
+    """sha256 (first 16 hex digits) of the STEP KERNEL sources (STEP_KERNEL_SOURCES; the host side of the ABI in
+    ukf_batch.cu and the per-filter access kernels do not change what a step executes) the library is built from:
+    profiles/traffic.json is stamped with it, so that ncu figures of an older kernel are not reported for a newer one.
+    Comments and white space do not count."""
     import hashlib
     import re
 
     h = hashlib.sha256()
-    for d in sorted(x for x in DEPS if x.endswith(".cuh")):
+    for d in sorted(STEP_KERNEL_SOURCES):
         with open(os.path.join(CSRC, d), "r") as f:
             code = re.sub(r"/\*.*?\*/|//[^\n]*", " ", f.read(), flags=re.S)
         h.update(d.encode() + b"\0" + " ".join(code.split()).encode())

@@ -78,6 +78,12 @@ SIGNATURES = {
     "ukfb_status_summary": (I, [P, C.POINTER(L), C.POINTER(C.c_uint32)]),
     "ukfb_get_mean_iter_hist": (I, [P, P]),
     "ukfb_clear_mean_iter_hist": (I, [P]),
+    "ukfb_get_state_indexed": (I, [P, L, P, P, P]),
+    "ukfb_get_state_indexed_dev": (I, [P, L, P, P, P]),
+    "ukfb_initialize_indexed": (I, [P, L, P, P, P]),
+    "ukfb_initialize_indexed_dev": (I, [P, L, P, P, P]),
+    "ukfb_find_status": (I, [P, C.c_uint32, L, P, C.POINTER(L)]),
+    "ukfb_clear_status_indexed": (I, [P, L, P]),
     "ukfb_synchronize": (I, [P]),
     "ukfb_stream": (P, [P]),
     "ukfb_event_record": (I, [P, I]),

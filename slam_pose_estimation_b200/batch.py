@@ -33,6 +33,8 @@ STATUS_BAD_EVENT, STATUS_MEAS_REJECTED = 32, 64
 
 RBS_DOUBLES = 49
 
+FIND_STATUS_FIRST = 1024  # matches UkfBatch.find_status fetches with the count
+
 ERR_INVALID, ERR_NOT_INITIALIZED, ERR_CUDA, ERR_NOMEM = -1, -2, -3, -4
 
 
@@ -58,6 +60,45 @@ def _dev(t):
     if not t.is_cuda or not t.is_contiguous():
         raise ValueError("device arguments must be contiguous CUDA tensors")
     return C.c_void_p(t.data_ptr())
+
+
+def _index_array(idx, who):
+    """a 1-D int64 array of filter indices (integer input of another width is widened; anything else is refused)"""
+    a = np.asarray(idx)
+    if a.ndim != 1:
+        raise ValueError(f"{who}: idx must be one-dimensional, got shape {a.shape}")
+    if a.size and not np.issubdtype(a.dtype, np.integer):
+        raise TypeError(f"{who}: idx must hold integers, got {a.dtype}")
+    a = np.ascontiguousarray(a, dtype=np.int64)
+    return a, a.ctypes.data_as(C.c_void_p)
+
+
+def _rows(a, shape, what):
+    """float64 rows of exactly `shape`, or the same flattened to one dimension"""
+    a = np.ascontiguousarray(a, dtype=np.float64)
+    if a.shape != tuple(shape) and a.shape != (int(np.prod(shape)),):
+        raise ValueError(f"{what} must be {shape}, got {a.shape}")
+    return a
+
+
+def _dev_index(t, who):
+    """number of indices in a device index tensor (int64, 1-D, contiguous)"""
+    if isinstance(t, int):
+        raise TypeError(f"{who}: pass the indices as a torch tensor (its length is the row count)")
+    import torch
+
+    if t.dtype != torch.int64 or t.dim() != 1:
+        raise TypeError(f"{who}: d_idx must be a 1-D int64 CUDA tensor, got {t.dtype} of shape {tuple(t.shape)}")
+    return int(t.numel())
+
+
+def _dev_rows(t, shape, what):
+    if isinstance(t, int):
+        return
+    import torch
+
+    if t.dtype != torch.float64 or tuple(t.shape) != tuple(shape):
+        raise ValueError(f"{what} must be a float64 CUDA tensor of shape {tuple(shape)}, got {t.dtype} {tuple(t.shape)}")
 
 
 def _torch_stream_of(*tensors):
@@ -402,6 +443,61 @@ class UkfBatch:
 
     def clear_mean_iter_hist(self):
         self._chk(self.lib.ukfb_clear_mean_iter_hist(self.h))
+
+    # ---- per-filter access -----------------------------------------------------------------------------
+    def get_state_indexed(self, idx, with_sigma: bool = True):
+        """getCurrentState of filters idx (global indices, any order, duplicates allowed): (mu n x MU, sigma n x n x n),
+        or mu alone with with_sigma=False.  Only those n rows travel."""
+        idx, pi = _index_array(idx, "get_state_indexed")
+        k = idx.size
+        mu = np.empty((k, self.MU))
+        sg = np.empty((k, self.n, self.n)) if with_sigma else None
+        self._chk(self.lib.ukfb_get_state_indexed(self.h, k, pi, mu.ctypes.data_as(C.c_void_p),
+                                                  sg.ctypes.data_as(C.c_void_p) if with_sigma else None))
+        return (mu, sg) if with_sigma else mu
+
+    def get_state_indexed_dev(self, d_idx, d_mu, d_sigma=None):
+        """the same into device tensors: d_idx int64 (n,), d_mu float64 (n, MU), d_sigma float64 (n, n, n) or None"""
+        k = _dev_index(d_idx, "get_state_indexed_dev")
+        _dev_rows(d_mu, (k, self.MU), "d_mu")
+        if d_sigma is not None:
+            _dev_rows(d_sigma, (k, self.n, self.n), "d_sigma")
+        self._after_torch(d_idx, d_mu, d_sigma)
+        self._chk(self.lib.ukfb_get_state_indexed_dev(self.h, k, _dev(d_idx), _dev(d_mu), _dev(d_sigma)))
+        self._before_torch(d_mu, d_sigma)
+
+    def initialize_indexed(self, idx, mu, sigma):
+        """initializeFilter of filters idx only (unique global indices): mu n x MU, sigma n x n x n; their t_last = 0.
+        Status words are left alone: clear_status_indexed after a recovery."""
+        idx, pi = _index_array(idx, "initialize_indexed")
+        k = idx.size
+        mu = _rows(mu, (k, self.MU), "mu")
+        sg = _rows(sigma, (k, self.n, self.n), "sigma")
+        self._chk(self.lib.ukfb_initialize_indexed(self.h, k, pi, mu.ctypes.data_as(C.c_void_p), sg.ctypes.data_as(C.c_void_p)))
+
+    def initialize_indexed_dev(self, d_idx, d_mu, d_sigma):
+        k = _dev_index(d_idx, "initialize_indexed_dev")
+        _dev_rows(d_mu, (k, self.MU), "d_mu")
+        _dev_rows(d_sigma, (k, self.n, self.n), "d_sigma")
+        self._after_torch(d_idx, d_mu, d_sigma)
+        self._chk(self.lib.ukfb_initialize_indexed_dev(self.h, k, _dev(d_idx), _dev(d_mu), _dev(d_sigma)))
+        self._before_torch(d_idx, d_mu, d_sigma)  # torch must not overwrite the inputs before the kernel has read them
+
+    def find_status(self, bits: int = 0xFFFFFFFF) -> np.ndarray:
+        """ascending indices of every filter whose status word has any of `bits`.  One call returns the count and the
+        first FIND_STATUS_FIRST matches (a few failed filters: one round trip); a second one fetches the rest."""
+        bits = int(bits) & 0xFFFFFFFF
+        n = C.c_int64()
+        out = np.empty(min(self.B, FIND_STATUS_FIRST), np.int64)
+        self._chk(self.lib.ukfb_find_status(self.h, bits, out.size, out.ctypes.data_as(C.c_void_p), C.byref(n)))
+        if n.value > out.size:
+            out = np.empty(n.value, np.int64)
+            self._chk(self.lib.ukfb_find_status(self.h, bits, n.value, out.ctypes.data_as(C.c_void_p), C.byref(n)))
+        return out[: n.value]
+
+    def clear_status_indexed(self, idx):
+        idx, pi = _index_array(idx, "clear_status_indexed")
+        self._chk(self.lib.ukfb_clear_status_indexed(self.h, idx.size, pi))
 
     # ---- stream plumbing ------------------------------------------------------------------------------
     def synchronize(self):

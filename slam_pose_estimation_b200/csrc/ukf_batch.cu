@@ -10,6 +10,7 @@
  */
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cfloat>
 #include <cmath>
 #include <vector>
@@ -26,6 +27,7 @@
 
 #include "ukf_device.cuh"
 #include "ukf_thread.cuh"
+#include "ukf_index.cuh"
 #ifndef UKFB_DEFAULT_PREFETCH_BYTES
 #define UKFB_DEFAULT_PREFETCH_BYTES 128
 #endif
@@ -257,12 +259,7 @@ static int fan_out(ukfb_handle* h, Fn fn)
 
 /* ---- small kernels ------------------------------------------------------------------------- */
 
-/* element index of record entry e of filter b: AoS records (warp kernel) or 32-filter entry-major tiles (thread kernel) */
-__device__ __forceinline__ long long rec_index(int tiled, long long b, int e, int REC)
-{
-    return tiled ? tile_index(b, e, REC) : b * REC + e;
-}
-
+/* rec_index (record entry e of filter b in either layout): ukf_index.cuh */
 
 /* host layout (mu B x MU, sigma B x n x n) -> records */
 __global__ void pack_kernel(double* __restrict__ state, const double* __restrict__ mu, const double* __restrict__ sigma,
@@ -1981,6 +1978,301 @@ extern "C" int ukfb_clear_mean_iter_hist(ukfb_handle* h)
     UKFB_FAN(h, ukfb_clear_mean_iter_hist(s_));
     CU(cudaMemsetAsync(h->hist, 0, sizeof(unsigned long long) * HIST_SLOTS * 8, h->stream));
     return UKFB_OK;
+}
+
+/* ---- per-filter access (kernels: ukf_index.cuh) ------------------------------------------------------------------ */
+static IndexParams index_params(const ukfb_handle* h, long long n_rows, const long long* d_idx)
+{
+    IndexParams p{};
+    p.state = h->state;
+    p.B = h->B;
+    p.MU = h->MU, p.n = h->n, p.REC = h->REC, p.tiled = h->tiled;
+    p.idx = d_idx;
+    p.n_rows = n_rows;
+    p.t_last = h->t_last;
+    p.status = h->status;
+    return p;
+}
+
+/* the checks of every host-pointer call, before anything is enqueued: indices in [0, B), unique when asked */
+static int check_indices(const ukfb_handle* h, int64_t n, const int64_t* idx, bool unique, const char* who)
+{
+    for (int64_t k = 0; k < n; ++k)
+        if (idx[k] < 0 || idx[k] >= h->B)
+            return fail(UKFB_ERR_INVALID, "%s: idx[%lld] = %lld is outside [0, %lld)", who, (long long)k, (long long)idx[k], h->B);
+    if (unique && n > 1) {
+        try {
+            std::vector<int64_t> s(idx, idx + n);
+            std::sort(s.begin(), s.end());
+            const auto d = std::adjacent_find(s.begin(), s.end());
+            if (d != s.end()) return fail(UKFB_ERR_INVALID, "%s: filter %lld is listed twice", who, (long long)*d);
+        } catch (const std::bad_alloc&) {
+            return fail(UKFB_ERR_NOMEM, "%s: out of host memory", who);
+        }
+    }
+    return UKFB_OK;
+}
+
+/* a sharded parent's index list split by shard: local indices and the caller's row of each, in the caller's order.
+ * Throws std::bad_alloc. */
+struct ShardRows {
+    std::vector<std::vector<int64_t>> local, pos;
+    ShardRows(const ukfb_handle* h, int64_t n, const int64_t* idx) : local(h->shards.size()), pos(h->shards.size())
+    {
+        for (int64_t k = 0; k < n; ++k) {
+            const size_t s = size_t(std::upper_bound(h->first.begin(), h->first.end(), (long long)idx[k]) - h->first.begin()) - 1;
+            local[s].push_back(idx[k] - h->first[s]);
+            pos[s].push_back(k);
+        }
+    }
+};
+
+/* the shard whose range starts at filter f (every shard holds at least one filter) */
+static size_t shard_at(const ukfb_handle* h, long long f)
+{
+    size_t i = 0;
+    while (h->first[i] != f) ++i;
+    return i;
+}
+
+static int get_state_indexed_launch(ukfb_handle* h, long long n, const long long* d_idx, double* d_mu, double* d_sigma)
+{
+    IndexParams p = index_params(h, n, d_idx);
+    p.mu = d_mu, p.sigma = d_sigma;
+    get_state_indexed_kernel<<<grid_for(n * (d_sigma ? h->n * h->n : h->MU)), 256, 0, h->stream>>>(p);
+    CU(cudaGetLastError());
+    return UKFB_OK;
+}
+
+extern "C" int ukfb_get_state_indexed_dev(ukfb_handle* h, int64_t n, const int64_t* d_idx, double* d_mu, double* d_sigma)
+{
+    CHECK_H(h);
+    UKFB_NOT_SHARDED(h);
+    if (n < 0) return fail(UKFB_ERR_INVALID, "ukfb_get_state_indexed_dev: n is negative");
+    if (n == 0) return UKFB_OK;
+    if (!d_idx || !d_mu) return fail(UKFB_ERR_INVALID, "ukfb_get_state_indexed_dev: null argument");
+    NEED_INIT(h);
+    return get_state_indexed_launch(h, n, reinterpret_cast<const long long*>(d_idx), d_mu, d_sigma);
+}
+
+/* one device, checked indices: stages n rows only */
+static int get_state_indexed_one(ukfb_handle* h, int64_t n, const int64_t* idx, double* mu, double* sigma)
+{
+    CHECK_H(h); /* a shard runs this on its worker thread: select its device there */
+    if (n == 0) return UKFB_OK;
+    const size_t bi = align256(sizeof(int64_t) * n), bm = align256(sizeof(double) * n * h->MU), bs = sizeof(double) * n * h->n * h->n;
+    int rc = stage_reserve(h, bi + bm + (sigma ? bs : 0));
+    if (rc) return rc;
+    long long* d_idx = reinterpret_cast<long long*>(h->stage);
+    double* d_mu = reinterpret_cast<double*>(h->stage + bi);
+    double* d_sigma = reinterpret_cast<double*>(h->stage + bi + bm);
+    CU(cudaMemcpyAsync(d_idx, idx, sizeof(int64_t) * n, cudaMemcpyHostToDevice, h->stream));
+    rc = get_state_indexed_launch(h, n, d_idx, d_mu, sigma ? d_sigma : nullptr);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(mu, d_mu, sizeof(double) * n * h->MU, cudaMemcpyDeviceToHost, h->stream));
+    if (sigma) CU(cudaMemcpyAsync(sigma, d_sigma, bs, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    return UKFB_OK;
+}
+
+extern "C" int ukfb_get_state_indexed(ukfb_handle* h, int64_t n, const int64_t* idx, double* mu, double* sigma)
+{
+    CHECK_H(h);
+    if (n < 0) return fail(UKFB_ERR_INVALID, "ukfb_get_state_indexed: n is negative");
+    if (n == 0) return UKFB_OK;
+    if (!idx || !mu) return fail(UKFB_ERR_INVALID, "ukfb_get_state_indexed: null argument");
+    NEED_INIT(h);
+    int rc = check_indices(h, n, idx, false, "ukfb_get_state_indexed");
+    if (rc || !is_sharded(h)) return rc ? rc : get_state_indexed_one(h, n, idx, mu, sigma);
+    /* sharded: each shard gathers its rows into a buffer of its own, then puts them at the caller's rows */
+    const size_t nn = size_t(h->n) * size_t(h->n);
+    try {
+        const ShardRows rows(h, n, idx);
+        std::vector<std::vector<double>> m(h->shards.size()), sg(h->shards.size());
+        for (size_t i = 0; i < h->shards.size(); ++i) {
+            m[i].resize(rows.local[i].size() * size_t(h->MU));
+            if (sigma) sg[i].resize(rows.local[i].size() * nn);
+        }
+        return fan_out(h, [&](ukfb_handle* s_, long long f_, long long) -> int {
+            const size_t i = shard_at(h, f_);
+            const int64_t c = int64_t(rows.local[i].size());
+            const int r = get_state_indexed_one(s_, c, rows.local[i].data(), m[i].data(), sigma ? sg[i].data() : nullptr);
+            if (r) return r;
+            for (int64_t j = 0; j < c; ++j) {
+                const size_t k = size_t(rows.pos[i][size_t(j)]);
+                std::memcpy(mu + k * h->MU, m[i].data() + size_t(j) * h->MU, sizeof(double) * h->MU);
+                if (sigma) std::memcpy(sigma + k * nn, sg[i].data() + size_t(j) * nn, sizeof(double) * nn);
+            }
+            return UKFB_OK;
+        });
+    } catch (const std::bad_alloc&) {
+        return fail(UKFB_ERR_NOMEM, "ukfb_get_state_indexed: out of host memory");
+    }
+}
+
+static int initialize_indexed_launch(ukfb_handle* h, long long n, const long long* d_idx, const double* d_mu, const double* d_sigma)
+{
+    IndexParams p = index_params(h, n, d_idx);
+    p.mu = const_cast<double*>(d_mu), p.sigma = const_cast<double*>(d_sigma); /* read only by this kernel */
+    initialize_indexed_kernel<<<grid_for(n * h->REC), 256, 0, h->stream>>>(p);
+    CU(cudaGetLastError());
+    return UKFB_OK;
+}
+
+extern "C" int ukfb_initialize_indexed_dev(ukfb_handle* h, int64_t n, const int64_t* d_idx, const double* d_mu, const double* d_sigma)
+{
+    CHECK_H(h);
+    UKFB_NOT_SHARDED(h);
+    if (n < 0) return fail(UKFB_ERR_INVALID, "ukfb_initialize_indexed_dev: n is negative");
+    if (n == 0) return UKFB_OK;
+    if (!d_idx || !d_mu || !d_sigma) return fail(UKFB_ERR_INVALID, "ukfb_initialize_indexed_dev: null argument");
+    NEED_INIT(h);
+    return initialize_indexed_launch(h, n, reinterpret_cast<const long long*>(d_idx), d_mu, d_sigma);
+}
+
+static int initialize_indexed_one(ukfb_handle* h, int64_t n, const int64_t* idx, const double* mu, const double* sigma)
+{
+    CHECK_H(h); /* a shard runs this on its worker thread: select its device there */
+    if (n == 0) return UKFB_OK;
+    const size_t bi = align256(sizeof(int64_t) * n), bm = align256(sizeof(double) * n * h->MU), bs = sizeof(double) * n * h->n * h->n;
+    int rc = stage_reserve(h, bi + bm + bs);
+    if (rc) return rc;
+    long long* d_idx = reinterpret_cast<long long*>(h->stage);
+    double* d_mu = reinterpret_cast<double*>(h->stage + bi);
+    double* d_sigma = reinterpret_cast<double*>(h->stage + bi + bm);
+    CU(cudaMemcpyAsync(d_idx, idx, sizeof(int64_t) * n, cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(d_mu, mu, sizeof(double) * n * h->MU, cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(d_sigma, sigma, bs, cudaMemcpyHostToDevice, h->stream));
+    rc = initialize_indexed_launch(h, n, d_idx, d_mu, d_sigma);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(h->stream));
+    return UKFB_OK;
+}
+
+extern "C" int ukfb_initialize_indexed(ukfb_handle* h, int64_t n, const int64_t* idx, const double* mu, const double* sigma)
+{
+    CHECK_H(h);
+    if (n < 0) return fail(UKFB_ERR_INVALID, "ukfb_initialize_indexed: n is negative");
+    if (n == 0) return UKFB_OK;
+    if (!idx || !mu || !sigma) return fail(UKFB_ERR_INVALID, "ukfb_initialize_indexed: null argument");
+    NEED_INIT(h);
+    int rc = check_indices(h, n, idx, true, "ukfb_initialize_indexed");
+    if (rc || !is_sharded(h)) return rc ? rc : initialize_indexed_one(h, n, idx, mu, sigma);
+    /* sharded: each shard gets contiguous copies of its rows */
+    const size_t nn = size_t(h->n) * size_t(h->n);
+    try {
+        const ShardRows rows(h, n, idx);
+        std::vector<std::vector<double>> m(h->shards.size()), sg(h->shards.size());
+        for (size_t i = 0; i < h->shards.size(); ++i) {
+            const size_t c = rows.local[i].size();
+            m[i].resize(c * size_t(h->MU));
+            sg[i].resize(c * nn);
+            for (size_t j = 0; j < c; ++j) {
+                const size_t k = size_t(rows.pos[i][j]);
+                std::memcpy(m[i].data() + j * h->MU, mu + k * h->MU, sizeof(double) * h->MU);
+                std::memcpy(sg[i].data() + j * nn, sigma + k * nn, sizeof(double) * nn);
+            }
+        }
+        return fan_out(h, [&](ukfb_handle* s_, long long f_, long long) -> int {
+            const size_t i = shard_at(h, f_);
+            return initialize_indexed_one(s_, int64_t(rows.local[i].size()), rows.local[i].data(), m[i].data(), sg[i].data());
+        });
+    } catch (const std::bad_alloc&) {
+        return fail(UKFB_ERR_NOMEM, "ukfb_initialize_indexed: out of host memory");
+    }
+}
+
+/* one device: every match counted, the first min(max_n, count) written to idx */
+static int find_status_one(ukfb_handle* h, uint32_t bits, int64_t max_n, int64_t* idx, int64_t* n_found)
+{
+    CHECK_H(h); /* a shard runs this on its worker thread: select its device there */
+    const long long chunks = (h->B + FS_CHUNK - 1) / FS_CHUNK;
+    const long long cap = max_n < h->B ? (long long)max_n : h->B;
+    const size_t bc = align256(sizeof(long long) * (chunks + 1));
+    int rc = stage_reserve(h, bc + sizeof(long long) * (cap > 0 ? cap : 1));
+    if (rc) return rc;
+    IndexParams p = index_params(h, chunks, nullptr);
+    p.bits = bits;
+    p.max_n = cap;
+    p.counts = reinterpret_cast<long long*>(h->stage);
+    p.out_idx = reinterpret_cast<long long*>(h->stage + bc);
+    const size_t smem = sizeof(long long) * TILE;
+    find_status_count_kernel<<<unsigned(chunks), TILE, smem, h->stream>>>(p);
+    find_status_scan_kernel<<<1, TILE, smem, h->stream>>>(p);
+    if (cap > 0) find_status_write_kernel<<<unsigned(chunks), TILE, smem, h->stream>>>(p);
+    CU(cudaGetLastError());
+    long long total = 0;
+    CU(cudaMemcpyAsync(&total, p.counts + chunks, sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    const long long got = total < cap ? total : cap;
+    if (got > 0) {
+        CU(cudaMemcpyAsync(idx, p.out_idx, sizeof(long long) * got, cudaMemcpyDeviceToHost, h->stream));
+        CU(cudaStreamSynchronize(h->stream));
+    }
+    *n_found = total;
+    return UKFB_OK;
+}
+
+extern "C" int ukfb_find_status(ukfb_handle* h, uint32_t bits, int64_t max_n, int64_t* idx, int64_t* n_found)
+{
+    CHECK_H(h);
+    if (max_n < 0 || !n_found || (max_n > 0 && !idx)) return fail(UKFB_ERR_INVALID, "ukfb_find_status: bad argument");
+    if (!is_sharded(h)) return find_status_one(h, bits, max_n, idx, n_found);
+    /* sharded: up to max_n from every shard, concatenated in shard order (ascending), truncated; counts summed */
+    try {
+        const size_t S = h->shards.size();
+        std::vector<std::vector<int64_t>> part(S);
+        std::vector<int64_t> cnt(S, 0);
+        for (size_t i = 0; i < S; ++i) part[i].resize(size_t(std::min<long long>(max_n, h->first[i + 1] - h->first[i])));
+        const int rc = fan_out(h, [&](ukfb_handle* s_, long long f_, long long) -> int {
+            const size_t i = shard_at(h, f_);
+            return find_status_one(s_, bits, int64_t(part[i].size()), part[i].data(), &cnt[i]);
+        });
+        if (rc) return rc;
+        int64_t total = 0, w = 0;
+        for (size_t i = 0; i < S; ++i) {
+            const int64_t got = std::min<int64_t>(cnt[i], int64_t(part[i].size()));
+            for (int64_t j = 0; j < got && w < max_n; ++j) idx[w++] = part[i][size_t(j)] + h->first[i];
+            total += cnt[i];
+        }
+        *n_found = total;
+        return UKFB_OK;
+    } catch (const std::bad_alloc&) {
+        return fail(UKFB_ERR_NOMEM, "ukfb_find_status: out of host memory");
+    }
+}
+
+static int clear_status_indexed_one(ukfb_handle* h, int64_t n, const int64_t* idx)
+{
+    CHECK_H(h); /* a shard runs this on its worker thread: select its device there */
+    if (n == 0) return UKFB_OK;
+    int rc = stage_reserve(h, sizeof(int64_t) * n);
+    if (rc) return rc;
+    long long* d_idx = reinterpret_cast<long long*>(h->stage);
+    CU(cudaMemcpyAsync(d_idx, idx, sizeof(int64_t) * n, cudaMemcpyHostToDevice, h->stream));
+    clear_status_indexed_kernel<<<grid_for(n), 256, 0, h->stream>>>(index_params(h, n, d_idx));
+    CU(cudaGetLastError());
+    CU(cudaStreamSynchronize(h->stream));
+    return UKFB_OK;
+}
+
+extern "C" int ukfb_clear_status_indexed(ukfb_handle* h, int64_t n, const int64_t* idx)
+{
+    CHECK_H(h);
+    if (n < 0) return fail(UKFB_ERR_INVALID, "ukfb_clear_status_indexed: n is negative");
+    if (n == 0) return UKFB_OK;
+    if (!idx) return fail(UKFB_ERR_INVALID, "ukfb_clear_status_indexed: null argument");
+    int rc = check_indices(h, n, idx, false, "ukfb_clear_status_indexed");
+    if (rc || !is_sharded(h)) return rc ? rc : clear_status_indexed_one(h, n, idx);
+    try {
+        const ShardRows rows(h, n, idx);
+        return fan_out(h, [&](ukfb_handle* s_, long long f_, long long) -> int {
+            const size_t i = shard_at(h, f_);
+            return clear_status_indexed_one(s_, int64_t(rows.local[i].size()), rows.local[i].data());
+        });
+    } catch (const std::bad_alloc&) {
+        return fail(UKFB_ERR_NOMEM, "ukfb_clear_status_indexed: out of host memory");
+    }
 }
 
 /* ---- stream plumbing ------------------------------------------------------------------------------------------ */
