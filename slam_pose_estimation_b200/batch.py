@@ -350,7 +350,8 @@ class UkfBatch:
         return out
 
     # ---- fused ------------------------------------------------------------------------------------
-    def step(self, dt, kind: int, mu=None, cov=None, mask=None):
+    def _step_args(self, dt, kind, mu, cov, mask):
+        """(the host arrays, which must outlive the call, and the arguments of ukfb_step after the handle)"""
         dt = np.atleast_1d(np.asarray(dt, np.float64))
         per = int(dt.size == self.B)
         dt, pd = _host(dt, np.float64)
@@ -358,20 +359,18 @@ class UkfBatch:
         cov, pc = _host(cov, np.float64)
         cper = 1 if (cov is not None and cov.ndim == 3) else 0
         mask, pk = _host(mask, np.uint8)
-        self._chk(self.lib.ukfb_step(self.h, pd, per, kind, pm, pc, cper, pk))
+        return (dt, mu, cov, mask), (pd, per, kind, pm, pc, cper, pk)
+
+    def step(self, dt, kind: int, mu=None, cov=None, mask=None):
+        arrays, args = self._step_args(dt, kind, mu, cov, mask)
+        self._chk(self.lib.ukfb_step(self.h, *args))
 
     def step_async(self, dt, kind: int, mu=None, cov=None, mask=None):
         """ukfb_step_async: enqueue only.  The arrays passed here are kept alive by this object until synchronize();
         pass pinned, C-contiguous float64 arrays (no conversion copy is made for those) for real overlap."""
-        dt = np.atleast_1d(np.asarray(dt, np.float64))
-        per = int(dt.size == self.B)
-        dt, pd = _host(dt, np.float64)
-        mu, pm = _host(mu, np.float64)
-        cov, pc = _host(cov, np.float64)
-        cper = 1 if (cov is not None and cov.ndim == 3) else 0
-        mask, pk = _host(mask, np.uint8)
-        self._inflight.append((dt, mu, cov, mask))
-        self._chk(self.lib.ukfb_step_async(self.h, pd, per, kind, pm, pc, cper, pk))
+        arrays, args = self._step_args(dt, kind, mu, cov, mask)
+        self._inflight.append(arrays)
+        self._chk(self.lib.ukfb_step_async(self.h, *args))
 
     def get_state_async(self, mu: np.ndarray, sigma: np.ndarray | None = None):
         """ukfb_get_state_async into caller-owned (pinned) host arrays; valid after synchronize()."""

@@ -11,6 +11,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cassert>
 #include <cfloat>
 #include <cmath>
 #include <vector>
@@ -128,21 +129,157 @@ struct ukfb_handle {
     } pipe;
 };
 
-static int stage_reserve(ukfb_handle* h, size_t bytes)
+static inline size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
+
+/* ---- host-pointer calls: device staging ---------------------------------------------------------------------------- */
+/* grows a staging buffer (h->stage, or a slot of h->pipe) to hold `bytes`, in whole MiB.  Whatever may still use the old
+ * buffer is waited for before it is freed: h->stream for h->stage, h->stream and both copy streams for a pipe slot. */
+static int stage_grow(ukfb_handle* h, char*& buf, size_t& have, size_t bytes, bool pipe_slot)
 {
-    if (bytes <= h->stage_bytes) return UKFB_OK;
+    if (bytes <= have) return UKFB_OK;
     CU(cudaStreamSynchronize(h->stream));
-    if (h->stage) CU(cudaFree(h->stage));
-    h->stage = nullptr;
-    h->stage_bytes = 0;
+    if (pipe_slot) {
+        CU(cudaStreamSynchronize(h->pipe.s_in));
+        CU(cudaStreamSynchronize(h->pipe.s_out));
+    }
+    if (buf) CU(cudaFree(buf));
+    buf = nullptr, have = 0;
     const size_t want = (bytes + (size_t(1) << 20)) & ~((size_t(1) << 20) - 1);
-    cudaError_t e = cudaMalloc(&h->stage, want);
-    if (e != cudaSuccess) return fail(UKFB_ERR_NOMEM, "staging buffer of %zu bytes: %s", want, cudaGetErrorString(e));
-    h->stage_bytes = want;
+    cudaError_t e = cudaMalloc(&buf, want);
+    if (e != cudaSuccess)
+        return fail(UKFB_ERR_NOMEM, "%sstaging buffer of %zu bytes: %s", pipe_slot ? "pipeline " : "", want, cudaGetErrorString(e));
+    have = want;
     return UKFB_OK;
 }
 
-static inline size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
+static int pipe_make(ukfb_handle* h)
+{
+    if (h->pipe.made) return UKFB_OK;
+    CU(cudaStreamCreateWithFlags(&h->pipe.s_in, cudaStreamNonBlocking));
+    CU(cudaStreamCreateWithFlags(&h->pipe.s_out, cudaStreamNonBlocking));
+    for (int i = 0; i < 2; ++i) {
+        CU(cudaEventCreateWithFlags(&h->pipe.in_ready[i], cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&h->pipe.in_consumed[i], cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&h->pipe.out_ready[i], cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&h->pipe.out_drained[i], cudaEventDisableTiming));
+    }
+    h->pipe.made = true;
+    return UKFB_OK;
+}
+
+/* The device side of one host-pointer call on one device.  The call registers every part first: in() / in_rows() copy
+ * host -> device, out() device -> host; a null host pointer skips its part and leaves its device pointer null.  Then
+ * commit() reserves the buffer ONCE for all parts -- growing it frees the old one, so no pointer into it may exist
+ * before --, sets the device pointers (256-byte aligned) and queues the host -> device copies.  After the call has
+ * enqueued its work on h->stream, finish() queues the device -> host copies and ends the call.
+ *   Blocking: h->stage, every copy on h->stream; finish() returns after cudaStreamSynchronize(h->stream).
+ *   Pipelined (the _async calls): one of two slots of h->pipe and no synchronisation, but where a slot grows.  A call
+ *   with inputs (ukfb_step_async, ukfb_run_events_async; counter pipe.n_in) copies them on s_in into slot n_in & 1 once
+ *   the launch that last read that slot is done (in_consumed), and its launch waits for the copies (in_ready).  A call
+ *   with outputs only (the _async getters; counter pipe.n_out) unpacks into slot n_out & 1 once the copies that last
+ *   read that slot are done (out_drained), and its copies on s_out wait for the unpack (out_ready).
+ * The host arrays of a pipelined call must stay valid and unchanged until ukfb_synchronize(). */
+struct Staging {
+    explicit Staging(ukfb_handle* h_, bool pipelined_) : h(h_), pipelined(pipelined_) {}
+
+    template <class T>
+    void in(T** dev, const void* src, size_t bytes) { add(dev, src, nullptr, bytes, 1, bytes); }
+    /* `rows` rows of `width` bytes, `pitch` bytes apart on the host (a shard's slice of slot-major K x B arrays), dense on
+     * the device */
+    template <class T>
+    void in_rows(T** dev, const void* src, size_t width, size_t rows, size_t pitch) { add(dev, src, nullptr, width, rows, pitch); }
+    template <class T>
+    void out(T** dev, void* dst, size_t bytes) { add(dev, nullptr, dst, bytes, 1, bytes); }
+
+    int commit()
+    {
+        size_t end = 0;
+        for (int i = 0; i < n; ++i) end = align256(end) + part[i].width * part[i].rows;
+        char* base;
+        if (!pipelined) {
+            if (int rc = stage_grow(h, h->stage, h->stage_bytes, end, false)) return rc;
+            base = h->stage;
+            cs = h->stream;
+        } else {
+            if (int rc = pipe_make(h)) return rc;
+            ukfb_handle::Pipe& p = h->pipe;
+            for (int i = 0; i < n; ++i) inputs = inputs || part[i].src;
+            slot = int((inputs ? p.n_in : p.n_out) & 1);
+            char*& buf = inputs ? p.in[slot] : p.out[slot];
+            if (int rc = stage_grow(h, buf, inputs ? p.in_bytes[slot] : p.out_bytes[slot], end, true)) return rc;
+            base = buf;
+            cs = inputs ? p.s_in : p.s_out;
+            if (inputs && p.n_in >= 2) CU(cudaStreamWaitEvent(cs, p.in_consumed[slot], 0)); /* the launch that read this slot is done */
+            if (!inputs && p.n_out >= 2) CU(cudaStreamWaitEvent(h->stream, p.out_drained[slot], 0)); /* the copies that read it are done */
+        }
+        size_t off = 0;
+        for (int i = 0; i < n; ++i) {
+            Part& q = part[i];
+            off = align256(off);
+            q.at = base + off;
+            off += q.width * q.rows;
+            q.set(q.dev, q.at);
+            if (q.src && q.width == q.pitch)
+                CU(cudaMemcpyAsync(q.at, q.src, q.width * q.rows, cudaMemcpyHostToDevice, cs));
+            else if (q.src)
+                CU(cudaMemcpy2DAsync(q.at, q.width, q.src, q.pitch, q.width, q.rows, cudaMemcpyHostToDevice, cs));
+        }
+        if (pipelined && inputs) {
+            CU(cudaEventRecord(h->pipe.in_ready[slot], cs));
+            CU(cudaStreamWaitEvent(h->stream, h->pipe.in_ready[slot], 0));
+        }
+        return UKFB_OK;
+    }
+
+    int finish()
+    {
+        ukfb_handle::Pipe& p = h->pipe;
+        if (pipelined && inputs) {
+            CU(cudaEventRecord(p.in_consumed[slot], h->stream));
+            p.n_in++;
+            return UKFB_OK;
+        }
+        if (pipelined) {
+            CU(cudaEventRecord(p.out_ready[slot], h->stream));
+            CU(cudaStreamWaitEvent(cs, p.out_ready[slot], 0));
+        }
+        for (int i = 0; i < n; ++i)
+            if (part[i].dst) CU(cudaMemcpyAsync(part[i].dst, part[i].at, part[i].width, cudaMemcpyDeviceToHost, cs));
+        if (!pipelined) {
+            CU(cudaStreamSynchronize(h->stream));
+            return UKFB_OK;
+        }
+        CU(cudaEventRecord(p.out_drained[slot], cs));
+        p.n_out++;
+        return UKFB_OK;
+    }
+
+private:
+    struct Part {
+        void* dev;                /* the caller's T* to set */
+        void (*set)(void*, char*); /* stores the device address into it as a T* */
+        const void* src;          /* host -> device */
+        void* dst;                /* device -> host */
+        size_t width, rows, pitch;
+        char* at;                 /* device address, from commit() on */
+    };
+    template <class T>
+    void add(T** dev, const void* src, void* dst, size_t width, size_t rows, size_t pitch)
+    {
+        *dev = nullptr;
+        if (!src && !dst) return;
+        assert(n < MAX_PARTS);
+        part[n++] = Part{dev, [](void* d, char* a) { *static_cast<T**>(d) = reinterpret_cast<T*>(a); }, src, dst, width, rows, pitch, nullptr};
+    }
+    static constexpr int MAX_PARTS = 4;
+    ukfb_handle* h;
+    bool pipelined;
+    bool inputs = false; /* pipelined: the call uses the input side of the pipe */
+    int slot = 0;
+    cudaStream_t cs = nullptr; /* the stream of the copies */
+    Part part[MAX_PARTS];
+    int n = 0;
+};
 
 struct Bind { /* sets the device for the duration of a call */
     int prev = -1;
@@ -158,10 +295,12 @@ struct Bind { /* sets the device for the duration of a call */
     }
 };
 
-#define CHECK_H(h)                                                      \
-    if (!(h)) return fail(UKFB_ERR_INVALID, "%s: null handle", __func__); \
-    Bind bind_(h);                                                      \
-    if (!bind_.ok) return fail(UKFB_ERR_CUDA, "%s: cudaSetDevice(%d) failed", __func__, (h)->device)
+/* `who`: the entry point named in the error text */
+#define CHECK_H_AS(h, who)                                                \
+    if (!(h)) return fail(UKFB_ERR_INVALID, "%s: null handle", who);      \
+    Bind bind_(h);                                                        \
+    if (!bind_.ok) return fail(UKFB_ERR_CUDA, "%s: cudaSetDevice(%d) failed", who, (h)->device)
+#define CHECK_H(h) CHECK_H_AS(h, __func__)
 
 /* ---- sharded handles: one worker thread per shard ---------------------------------------------------------------- */
 /* Filters share nothing (UnscentedKalmanFilter.hpp:150-154), so a sharded parent is just a list of one-device handles
@@ -714,8 +853,9 @@ static bool kind_ok(const ukfb_handle* h, int kind)
     return kind == UKFB_MEAS_ORI_VELOCITY;
 }
 
-#define NEED_INIT(h) \
-    if (!(h)->initialized) return fail(UKFB_ERR_NOT_INITIALIZED, "%s: filter not initialized", __func__)
+#define NEED_INIT_AS(h, who) \
+    if (!(h)->initialized) return fail(UKFB_ERR_NOT_INITIALIZED, "%s: filter not initialized", who)
+#define NEED_INIT(h) NEED_INIT_AS(h, __func__)
 
 /* ---- lifecycle ---------------------------------------------------------------------------------- */
 extern "C" int ukfb_create(int filter_kind, int64_t batch, int device, ukfb_handle** out)
@@ -937,17 +1077,13 @@ extern "C" int ukfb_initialize(ukfb_handle* h, const double* mu, const double* s
         if (rc == UKFB_OK) h->initialized = true;
         return rc;
     }
-    const size_t bm = align256(sizeof(double) * h->B * h->MU), bs = sizeof(double) * h->B * h->n * h->n;
-    int rc = stage_reserve(h, bm + bs);
-    if (rc) return rc;
-    double* d_mu = reinterpret_cast<double*>(h->stage);
-    double* d_sigma = reinterpret_cast<double*>(h->stage + bm);
-    CU(cudaMemcpyAsync(d_mu, mu, sizeof(double) * h->B * h->MU, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(d_sigma, sigma, bs, cudaMemcpyHostToDevice, h->stream));
-    rc = initialize_dev(h, d_mu, d_sigma);
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    const double *d_mu, *d_sigma;
+    Staging st(h, false);
+    st.in(&d_mu, mu, sizeof(double) * h->B * h->MU);
+    st.in(&d_sigma, sigma, sizeof(double) * h->B * h->n * h->n);
+    int rc = st.commit();
+    if (!rc) rc = initialize_dev(h, d_mu, d_sigma);
+    return rc ? rc : st.finish();
 }
 
 extern "C" int ukfb_initialize_from_body_states_dev(ukfb_handle* h, const double* d_rbs)
@@ -974,14 +1110,12 @@ extern "C" int ukfb_initialize_from_body_states(ukfb_handle* h, const double* rb
         if (rc == UKFB_OK) h->initialized = true;
         return rc;
     }
-    const size_t bytes = sizeof(double) * h->B * UKFB_RBS_DOUBLES;
-    int rc = stage_reserve(h, bytes);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(h->stage, rbs, bytes, cudaMemcpyHostToDevice, h->stream));
-    rc = ukfb_initialize_from_body_states_dev(h, reinterpret_cast<const double*>(h->stage));
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    const double* d_rbs;
+    Staging st(h, false);
+    st.in(&d_rbs, rbs, sizeof(double) * h->B * UKFB_RBS_DOUBLES);
+    int rc = st.commit();
+    if (!rc) rc = ukfb_initialize_from_body_states_dev(h, d_rbs);
+    return rc ? rc : st.finish();
 }
 
 extern "C" int ukfb_get_body_states_dev(ukfb_handle* h, double* d_rbs)
@@ -1002,14 +1136,12 @@ extern "C" int ukfb_get_body_states(ukfb_handle* h, double* rbs)
     NEED_INIT(h);
     if (!rbs) return fail(UKFB_ERR_INVALID, "ukfb_get_body_states: null argument");
     UKFB_FAN(h, ukfb_get_body_states(s_, rbs + f_ * UKFB_RBS_DOUBLES));
-    const size_t bytes = sizeof(double) * h->B * UKFB_RBS_DOUBLES;
-    int rc = stage_reserve(h, bytes);
-    if (rc) return rc;
-    rc = ukfb_get_body_states_dev(h, reinterpret_cast<double*>(h->stage));
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(rbs, h->stage, bytes, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    double* d_rbs;
+    Staging st(h, false);
+    st.out(&d_rbs, rbs, sizeof(double) * h->B * UKFB_RBS_DOUBLES);
+    int rc = st.commit();
+    if (!rc) rc = ukfb_get_body_states_dev(h, d_rbs);
+    return rc ? rc : st.finish();
 }
 
 extern "C" int ukfb_get_state_dev(ukfb_handle* h, double* d_mu, double* d_sigma)
@@ -1023,23 +1155,33 @@ extern "C" int ukfb_get_state_dev(ukfb_handle* h, double* d_mu, double* d_sigma)
     return UKFB_OK;
 }
 
+/* ukfb_get_state / ukfb_get_state_async */
+static int get_state_host(ukfb_handle* h, double* mu, double* sigma, bool pipelined, const char* who)
+{
+    CHECK_H_AS(h, who);
+    NEED_INIT_AS(h, who);
+    /* sharded: every shard lands in its range of the caller's single buffer -- the final gather of the estimates */
+    UKFB_FAN(h, get_state_host(s_, mu ? mu + f_ * s_->MU : nullptr, sigma ? sigma + f_ * s_->n * s_->n : nullptr, pipelined, who));
+    double *d_mu, *d_sigma;
+    Staging st(h, pipelined);
+    st.out(&d_mu, mu, sizeof(double) * h->B * h->MU);
+    st.out(&d_sigma, sigma, sizeof(double) * h->B * h->n * h->n);
+    int rc = st.commit();
+    if (!rc) rc = ukfb_get_state_dev(h, d_mu, d_sigma);
+    return rc ? rc : st.finish();
+}
+
 extern "C" int ukfb_get_state(ukfb_handle* h, double* mu, double* sigma)
 {
-    CHECK_H(h);
-    NEED_INIT(h);
-    /* sharded: every shard lands in its range of the caller's single buffer -- the final gather of the estimates */
-    UKFB_FAN(h, ukfb_get_state(s_, mu ? mu + f_ * s_->MU : nullptr, sigma ? sigma + f_ * s_->n * s_->n : nullptr));
-    const size_t bm = align256(sizeof(double) * h->B * h->MU), bs = sizeof(double) * h->B * h->n * h->n;
-    int rc = stage_reserve(h, bm + (sigma ? bs : 0));
-    if (rc) return rc;
-    double* d_mu = reinterpret_cast<double*>(h->stage);
-    double* d_sigma = reinterpret_cast<double*>(h->stage + bm);
-    rc = ukfb_get_state_dev(h, mu ? d_mu : nullptr, sigma ? d_sigma : nullptr);
-    if (rc) return rc;
-    if (mu) CU(cudaMemcpyAsync(mu, d_mu, sizeof(double) * h->B * h->MU, cudaMemcpyDeviceToHost, h->stream));
-    if (sigma) CU(cudaMemcpyAsync(sigma, d_sigma, bs, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    return get_state_host(h, mu, sigma, false, "ukfb_get_state");
+}
+
+/* ukfb_get_state without the final synchronisation: the estimates of the steps issued so far are unpacked on the
+ * compute stream into one of two staging slots and copied to the host on a copy-out stream, overlapping later
+ * steps; mu / sigma are valid after ukfb_synchronize(). */
+extern "C" int ukfb_get_state_async(ukfb_handle* h, double* mu, double* sigma)
+{
+    return get_state_host(h, mu, sigma, true, "ukfb_get_state_async");
 }
 
 /* mu entries [first, first + count) of every filter, dense B x count */
@@ -1073,21 +1215,30 @@ extern "C" int ukfb_get_mu_range_dev(ukfb_handle* h, int mu_first, int mu_count,
     return UKFB_OK;
 }
 
+/* ukfb_get_mu_range / ukfb_get_mu_range_async */
+static int get_mu_range_host(ukfb_handle* h, int mu_first, int mu_count, double* out, bool pipelined, const char* who)
+{
+    CHECK_H_AS(h, who);
+    NEED_INIT_AS(h, who);
+    int rc = mu_range_ok(h, mu_first, mu_count, out, who);
+    if (rc) return rc;
+    UKFB_FAN(h, get_mu_range_host(s_, mu_first, mu_count, out + f_ * mu_count, pipelined, who));
+    double* d_out;
+    Staging st(h, pipelined);
+    st.out(&d_out, out, sizeof(double) * h->B * mu_count);
+    rc = st.commit();
+    if (!rc) rc = ukfb_get_mu_range_dev(h, mu_first, mu_count, d_out);
+    return rc ? rc : st.finish();
+}
+
 extern "C" int ukfb_get_mu_range(ukfb_handle* h, int mu_first, int mu_count, double* out)
 {
-    CHECK_H(h);
-    NEED_INIT(h);
-    int rc = mu_range_ok(h, mu_first, mu_count, out, "ukfb_get_mu_range");
-    if (rc) return rc;
-    UKFB_FAN(h, ukfb_get_mu_range(s_, mu_first, mu_count, out + f_ * mu_count));
-    const size_t bytes = sizeof(double) * h->B * mu_count;
-    rc = stage_reserve(h, bytes);
-    if (rc) return rc;
-    rc = ukfb_get_mu_range_dev(h, mu_first, mu_count, reinterpret_cast<double*>(h->stage));
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(out, h->stage, bytes, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    return get_mu_range_host(h, mu_first, mu_count, out, false, "ukfb_get_mu_range");
+}
+
+extern "C" int ukfb_get_mu_range_async(ukfb_handle* h, int mu_first, int mu_count, double* out)
+{
+    return get_mu_range_host(h, mu_first, mu_count, out, true, "ukfb_get_mu_range_async");
 }
 
 extern "C" int ukfb_set_process_noise(ukfb_handle* h, const double* Q, int per_filter)
@@ -1096,11 +1247,13 @@ extern "C" int ukfb_set_process_noise(ukfb_handle* h, const double* Q, int per_f
     if (!Q) return fail(UKFB_ERR_INVALID, "ukfb_set_process_noise: null argument");
     UKFB_FAN(h, ukfb_set_process_noise(s_, Q + (per_filter ? f_ * s_->n * s_->n : 0), per_filter));
     const long long count = per_filter ? h->B : 1;
-    const size_t bytes = sizeof(double) * count * h->n * h->n;
-    int rc = stage_reserve(h, bytes);
+    const double* d_Q;
+    Staging st(h, false);
+    st.in(&d_Q, Q, sizeof(double) * count * h->n * h->n);
+    int rc = st.commit();
     if (rc) return rc;
     if ((per_filter != 0) != (h->q_per_filter != 0)) {
-        CU(cudaStreamSynchronize(h->stream));
+        CU(cudaStreamSynchronize(h->stream)); /* also completes the copy of Q queued above: a failure below leaves nothing reading Q */
         double* nq = nullptr;
         cudaError_t e = cudaMalloc(&nq, sizeof(double) * count * h->LP);
         if (e != cudaSuccess) return fail(UKFB_ERR_NOMEM, "ukfb_set_process_noise: %s", cudaGetErrorString(e));
@@ -1118,11 +1271,9 @@ extern "C" int ukfb_set_process_noise(ukfb_handle* h, const double* Q, int per_f
         if (h->q_diagonal && Q[0] == Q[n + 1] && Q[0] == Q[2 * n + 2] && Q[3 * n + 3] == Q[4 * n + 4] && Q[3 * n + 3] == Q[5 * n + 5])
             h->q_diagonal = 2;
     }
-    CU(cudaMemcpyAsync(h->stage, Q, bytes, cudaMemcpyHostToDevice, h->stream));
-    pack_q_kernel<<<grid_for(count * h->LP), 256, 0, h->stream>>>(h->Q, reinterpret_cast<const double*>(h->stage), count, h->n, h->LP);
+    pack_q_kernel<<<grid_for(count * h->LP), 256, 0, h->stream>>>(h->Q, d_Q, count, h->n, h->LP);
     CU(cudaGetLastError());
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    return st.finish();
 }
 
 extern "C" int ukfb_get_process_noise(ukfb_handle* h, double* Q, int per_filter)
@@ -1131,15 +1282,14 @@ extern "C" int ukfb_get_process_noise(ukfb_handle* h, double* Q, int per_filter)
     if (!Q) return fail(UKFB_ERR_INVALID, "ukfb_get_process_noise: null argument");
     UKFB_FAN(h, (per_filter || f_ == 0) ? ukfb_get_process_noise(s_, Q + (per_filter ? f_ * s_->n * s_->n : 0), per_filter) : UKFB_OK);
     const long long count = per_filter ? h->B : 1;
-    const size_t bytes = sizeof(double) * count * h->n * h->n;
-    int rc = stage_reserve(h, bytes);
+    double* d_Q;
+    Staging st(h, false);
+    st.out(&d_Q, Q, sizeof(double) * count * h->n * h->n);
+    int rc = st.commit();
     if (rc) return rc;
-    unpack_q_kernel<<<grid_for(count * h->n * h->n), 256, 0, h->stream>>>(h->Q, reinterpret_cast<double*>(h->stage), count, h->n, h->LP,
-                                                                         h->q_per_filter ? h->LP : 0);
+    unpack_q_kernel<<<grid_for(count * h->n * h->n), 256, 0, h->stream>>>(h->Q, d_Q, count, h->n, h->LP, h->q_per_filter ? h->LP : 0);
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(Q, h->stage, bytes, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    return st.finish();
 }
 
 extern "C" int ukfb_set_time_bounds(ukfb_handle* h, double min_dt, double max_dt)
@@ -1268,14 +1418,12 @@ extern "C" int ukfb_predict_dt(ukfb_handle* h, const double* dt, int per_filter)
     NEED_INIT(h);
     if (!dt) return fail(UKFB_ERR_INVALID, "ukfb_predict_dt: null argument");
     UKFB_FAN(h, ukfb_predict_dt(s_, dt + (per_filter ? f_ : 0), per_filter));
-    const size_t bytes = sizeof(double) * (per_filter ? h->B : 1);
-    int rc = stage_reserve(h, bytes);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(h->stage, dt, bytes, cudaMemcpyHostToDevice, h->stream));
-    rc = ukfb_predict_dt_dev(h, reinterpret_cast<const double*>(h->stage), per_filter);
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    const double* d_dt;
+    Staging st(h, false);
+    st.in(&d_dt, dt, sizeof(double) * (per_filter ? h->B : 1));
+    int rc = st.commit();
+    if (!rc) rc = ukfb_predict_dt_dev(h, d_dt, per_filter);
+    return rc ? rc : st.finish();
 }
 
 extern "C" int ukfb_predict_time_dev(ukfb_handle* h, const int64_t* d_ts_us, int per_filter)
@@ -1298,14 +1446,12 @@ extern "C" int ukfb_predict_time(ukfb_handle* h, const int64_t* ts_us, int per_f
     NEED_INIT(h);
     if (!ts_us) return fail(UKFB_ERR_INVALID, "ukfb_predict_time: null argument");
     UKFB_FAN(h, ukfb_predict_time(s_, ts_us + (per_filter ? f_ : 0), per_filter));
-    const size_t bytes = sizeof(int64_t) * (per_filter ? h->B : 1);
-    int rc = stage_reserve(h, bytes);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(h->stage, ts_us, bytes, cudaMemcpyHostToDevice, h->stream));
-    rc = ukfb_predict_time_dev(h, reinterpret_cast<const int64_t*>(h->stage), per_filter);
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    const int64_t* d_ts;
+    Staging st(h, false);
+    st.in(&d_ts, ts_us, sizeof(int64_t) * (per_filter ? h->B : 1));
+    int rc = st.commit();
+    if (!rc) rc = ukfb_predict_time_dev(h, d_ts, per_filter);
+    return rc ? rc : st.finish();
 }
 
 /* ---- measurements ------------------------------------------------------------------------------------ */
@@ -1341,39 +1487,6 @@ extern "C" int ukfb_update_dev(ukfb_handle* h, int meas_kind, const double* d_mu
     return launch_step(h, p);
 }
 
-/* copies (mu, cov, mask) of one measurement into the staging buffer at `off`; returns device pointers */
-static int stage_meas(ukfb_handle* h, size_t off, int m, const double* mu, const double* cov, int cov_per_filter, const uint8_t* mask,
-                      const double** d_mu, const double** d_cov, const uint8_t** d_mask, size_t* end)
-{
-    const size_t bm = align256(sizeof(double) * h->B * m);
-    const size_t bc = cov ? align256(sizeof(double) * (cov_per_filter ? h->B : 1) * m * m) : 0;
-    const size_t bk = mask ? align256(size_t(h->B)) : 0;
-    int rc = stage_reserve(h, off + bm + bc + bk);
-    if (rc) return rc;
-    char* base = h->stage + off;
-    CU(cudaMemcpyAsync(base, mu, sizeof(double) * h->B * m, cudaMemcpyHostToDevice, h->stream));
-    *d_mu = reinterpret_cast<const double*>(base);
-    *d_cov = nullptr;
-    if (cov) {
-        CU(cudaMemcpyAsync(base + bm, cov, sizeof(double) * (cov_per_filter ? h->B : 1) * m * m, cudaMemcpyHostToDevice, h->stream));
-        *d_cov = reinterpret_cast<const double*>(base + bm);
-    }
-    *d_mask = nullptr;
-    if (mask) {
-        CU(cudaMemcpyAsync(base + bm + bc, mask, size_t(h->B), cudaMemcpyHostToDevice, h->stream));
-        *d_mask = reinterpret_cast<const uint8_t*>(base + bm + bc);
-    }
-    if (end) *end = off + bm + bc + bk;
-    return UKFB_OK;
-}
-
-/* the staging buffer must be large enough BEFORE pointers into it are taken */
-static size_t meas_bytes(const ukfb_handle* h, int m, bool cov, int cov_per_filter, bool mask)
-{
-    return align256(sizeof(double) * h->B * m) + (cov ? align256(sizeof(double) * (cov_per_filter ? h->B : 1) * m * m) : 0) +
-           (mask ? align256(size_t(h->B)) : 0);
-}
-
 extern "C" int ukfb_update(ukfb_handle* h, int meas_kind, const double* mu, const double* cov, int cov_per_filter, const uint8_t* mask)
 {
     CHECK_H(h);
@@ -1385,13 +1498,15 @@ extern "C" int ukfb_update(ukfb_handle* h, int meas_kind, const double* mu, cons
     UKFB_FAN(h, ukfb_update(s_, meas_kind, mu + f_ * m, cov ? cov + (cov_per_filter ? f_ * m * m : 0) : nullptr, cov_per_filter, mask ? mask + f_ : nullptr));
     const double *d_mu, *d_cov;
     const uint8_t* d_mask;
-    int rc = stage_meas(h, 0, m, mu, cov, cov_per_filter, mask, &d_mu, &d_cov, &d_mask, nullptr);
+    Staging st(h, false);
+    st.in(&d_mu, mu, sizeof(double) * h->B * m);
+    st.in(&d_cov, cov, sizeof(double) * (cov_per_filter ? h->B : 1) * m * m);
+    st.in(&d_mask, mask, size_t(h->B));
+    int rc = st.commit();
     if (rc) return rc;
     if (!cov) d_cov = h->meas_cov[meas_kind], cov_per_filter = h->meas_cov_per_filter[meas_kind] == 2;
     rc = ukfb_update_dev(h, meas_kind, d_mu, d_cov, cov_per_filter, d_mask);
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    return rc ? rc : st.finish();
 }
 
 extern "C" int ukfb_set_measurement_cov(ukfb_handle* h, int meas_kind, const double* cov, int per_filter)
@@ -1445,17 +1560,15 @@ extern "C" int ukfb_update_mixed(ukfb_handle* h, const int8_t* kinds, const doub
         if (kinds[b] != UKFB_MEAS_NONE && !kind_ok(h, kinds[b]))
             return fail(UKFB_ERR_INVALID, "ukfb_update_mixed: kinds[%lld] = %d does not belong to this filter kind", b, int(kinds[b]));
     UKFB_FAN(h, ukfb_update_mixed(s_, kinds + f_, mu3 + f_ * 3, cov33 + f_ * 9));
-    const size_t bk = align256(size_t(h->B)), bm = align256(sizeof(double) * h->B * 3), bc = sizeof(double) * h->B * 9;
-    int rc = stage_reserve(h, bk + bm + bc);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(h->stage, kinds, size_t(h->B), cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(h->stage + bk, mu3, sizeof(double) * h->B * 3, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(h->stage + bk + bm, cov33, bc, cudaMemcpyHostToDevice, h->stream));
-    rc = ukfb_update_mixed_dev(h, reinterpret_cast<const int8_t*>(h->stage), reinterpret_cast<const double*>(h->stage + bk),
-                               reinterpret_cast<const double*>(h->stage + bk + bm));
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    const int8_t* d_kinds;
+    const double *d_mu3, *d_cov33;
+    Staging st(h, false);
+    st.in(&d_kinds, kinds, size_t(h->B));
+    st.in(&d_mu3, mu3, sizeof(double) * h->B * 3);
+    st.in(&d_cov33, cov33, sizeof(double) * h->B * 9);
+    int rc = st.commit();
+    if (!rc) rc = ukfb_update_mixed_dev(h, d_kinds, d_mu3, d_cov33);
+    return rc ? rc : st.finish();
 }
 
 static int store_vec3_dev(ukfb_handle* h, double* dst_mu, double* dst_cov, const double* d_mu, const double* d_cov, int cov_per_filter,
@@ -1482,12 +1595,13 @@ extern "C" int ukfb_set_acceleration(ukfb_handle* h, const double* mu, const dou
     UKFB_FAN(h, ukfb_set_acceleration(s_, mu + f_ * 3, cov ? cov + (cov_per_filter ? f_ * 9 : 0) : nullptr, cov_per_filter, mask ? mask + f_ : nullptr));
     const double *d_mu, *d_cov;
     const uint8_t* d_mask;
-    int rc = stage_meas(h, 0, 3, mu, cov, cov_per_filter, mask, &d_mu, &d_cov, &d_mask, nullptr);
-    if (rc) return rc;
-    rc = ukfb_set_acceleration_dev(h, d_mu, d_cov, cov_per_filter, d_mask);
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    Staging st(h, false);
+    st.in(&d_mu, mu, sizeof(double) * h->B * 3);
+    st.in(&d_cov, cov, sizeof(double) * (cov_per_filter ? h->B : 1) * 9);
+    st.in(&d_mask, mask, size_t(h->B));
+    int rc = st.commit();
+    if (!rc) rc = ukfb_set_acceleration_dev(h, d_mu, d_cov, cov_per_filter, d_mask);
+    return rc ? rc : st.finish();
 }
 
 extern "C" int ukfb_set_rotation_rate_dev(ukfb_handle* h, const double* d_mu, const double* d_cov, int cov_per_filter, const uint8_t* d_mask)
@@ -1509,12 +1623,13 @@ extern "C" int ukfb_set_rotation_rate(ukfb_handle* h, const double* mu, const do
     UKFB_FAN(h, ukfb_set_rotation_rate(s_, mu + f_ * 3, cov ? cov + (cov_per_filter ? f_ * 9 : 0) : nullptr, cov_per_filter, mask ? mask + f_ : nullptr));
     const double *d_mu, *d_cov;
     const uint8_t* d_mask;
-    int rc = stage_meas(h, 0, 3, mu, cov, cov_per_filter, mask, &d_mu, &d_cov, &d_mask, nullptr);
-    if (rc) return rc;
-    rc = ukfb_set_rotation_rate_dev(h, d_mu, d_cov, cov_per_filter, d_mask);
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    Staging st(h, false);
+    st.in(&d_mu, mu, sizeof(double) * h->B * 3);
+    st.in(&d_cov, cov, sizeof(double) * (cov_per_filter ? h->B : 1) * 9);
+    st.in(&d_mask, mask, size_t(h->B));
+    int rc = st.commit();
+    if (!rc) rc = ukfb_set_rotation_rate_dev(h, d_mu, d_cov, cov_per_filter, d_mask);
+    return rc ? rc : st.finish();
 }
 
 extern "C" int ukfb_get_rotation_rate(ukfb_handle* h, double* out)
@@ -1524,14 +1639,15 @@ extern "C" int ukfb_get_rotation_rate(ukfb_handle* h, double* out)
     if (h->kind != UKFB_ORIENTATION) return fail(UKFB_ERR_INVALID, "ukfb_get_rotation_rate: not an ORIENTATION handle");
     if (!out) return fail(UKFB_ERR_INVALID, "ukfb_get_rotation_rate: null argument");
     UKFB_FAN(h, ukfb_get_rotation_rate(s_, out + f_ * 3));
-    int rc = stage_reserve(h, sizeof(double) * h->B * 3);
+    double* d_out;
+    Staging st(h, false);
+    st.out(&d_out, out, sizeof(double) * h->B * 3);
+    int rc = st.commit();
     if (rc) return rc;
     rotation_rate_kernel<<<grid_for(h->B), 256, 0, h->stream>>>(h->state, h->gyro_mu, h->earth[0], h->earth[1], h->earth[2], h->ori_params,
-                                                               reinterpret_cast<double*>(h->stage), h->B, h->tiled);
+                                                               d_out, h->B, h->tiled);
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(out, h->stage, sizeof(double) * h->B * 3, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    return st.finish();
 }
 
 /* ---- fused step ------------------------------------------------------------------------------------------ */
@@ -1554,65 +1670,41 @@ extern "C" int ukfb_step_dev(ukfb_handle* h, const double* d_dt, int dt_per_filt
     return launch_step(h, p);
 }
 
+/* ukfb_step / ukfb_step_async */
+static int step_host(ukfb_handle* h, const double* dt, int dt_per_filter, int meas_kind, const double* mu, const double* cov,
+                     int cov_per_filter, const uint8_t* mask, bool pipelined, const char* who)
+{
+    CHECK_H_AS(h, who);
+    NEED_INIT_AS(h, who);
+    if (!dt) return fail(UKFB_ERR_INVALID, "%s: null dt", who);
+    const bool upd = meas_kind != UKFB_MEAS_NONE;
+    if (upd && !kind_ok(h, meas_kind)) return fail(UKFB_ERR_INVALID, "%s: measurement kind %d does not belong to this filter kind", who, meas_kind);
+    if (upd && !mu) return fail(UKFB_ERR_INVALID, "%s: null measurement", who);
+    if (upd && !cov && !h->meas_cov_per_filter[meas_kind])
+        return fail(UKFB_ERR_INVALID, "%s: null covariance and none kept by ukfb_set_measurement_cov for kind %d", who, meas_kind);
+    const int m = upd ? meas_dim(meas_kind) : 0;
+    UKFB_FAN(h, step_host(s_, dt + (dt_per_filter ? f_ : 0), dt_per_filter, meas_kind, mu ? mu + f_ * m : nullptr,
+                          cov ? cov + (cov_per_filter ? f_ * m * m : 0) : nullptr, cov_per_filter, mask ? mask + f_ : nullptr, pipelined, who));
+    const double *d_dt, *d_mu = nullptr, *d_cov = nullptr;
+    const uint8_t* d_mask = nullptr;
+    Staging st(h, pipelined);
+    st.in(&d_dt, dt, sizeof(double) * (dt_per_filter ? h->B : 1));
+    if (upd) {
+        st.in(&d_mu, mu, sizeof(double) * h->B * m);
+        st.in(&d_cov, cov, sizeof(double) * (cov_per_filter ? h->B : 1) * m * m);
+        st.in(&d_mask, mask, size_t(h->B));
+    }
+    int rc = st.commit();
+    if (rc) return rc;
+    if (upd && !cov) d_cov = h->meas_cov[meas_kind], cov_per_filter = h->meas_cov_per_filter[meas_kind] == 2;
+    rc = ukfb_step_dev(h, d_dt, dt_per_filter, meas_kind, d_mu, d_cov, cov_per_filter, d_mask);
+    return rc ? rc : st.finish();
+}
+
 extern "C" int ukfb_step(ukfb_handle* h, const double* dt, int dt_per_filter, int meas_kind, const double* mu, const double* cov,
                          int cov_per_filter, const uint8_t* mask)
 {
-    CHECK_H(h);
-    NEED_INIT(h);
-    if (!dt) return fail(UKFB_ERR_INVALID, "ukfb_step: null dt");
-    const size_t bd = align256(sizeof(double) * (dt_per_filter ? h->B : 1));
-    const bool upd = meas_kind != UKFB_MEAS_NONE;
-    if (upd && !kind_ok(h, meas_kind)) return fail(UKFB_ERR_INVALID, "ukfb_step: measurement kind %d does not belong to this filter kind", meas_kind);
-    if (upd && !mu) return fail(UKFB_ERR_INVALID, "ukfb_step: null measurement");
-    if (upd && !cov && !h->meas_cov_per_filter[meas_kind]) return fail(UKFB_ERR_INVALID, "ukfb_step: null covariance and none kept by ukfb_set_measurement_cov for kind %d", meas_kind);
-    const int m = upd ? meas_dim(meas_kind) : 0;
-    UKFB_FAN(h, ukfb_step(s_, dt + (dt_per_filter ? f_ : 0), dt_per_filter, meas_kind, mu ? mu + f_ * m : nullptr,
-                          cov ? cov + (cov_per_filter ? f_ * m * m : 0) : nullptr, cov_per_filter, mask ? mask + f_ : nullptr));
-    int rc = stage_reserve(h, bd + (upd ? meas_bytes(h, m, cov != nullptr, cov_per_filter, mask != nullptr) : 0));
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(h->stage, dt, sizeof(double) * (dt_per_filter ? h->B : 1), cudaMemcpyHostToDevice, h->stream));
-    const double *d_mu = nullptr, *d_cov = nullptr;
-    const uint8_t* d_mask = nullptr;
-    if (upd) {
-        rc = stage_meas(h, bd, m, mu, cov, cov_per_filter, mask, &d_mu, &d_cov, &d_mask, nullptr);
-        if (rc) return rc;
-        if (!cov) d_cov = h->meas_cov[meas_kind], cov_per_filter = h->meas_cov_per_filter[meas_kind] == 2;
-    }
-    rc = ukfb_step_dev(h, reinterpret_cast<const double*>(h->stage), dt_per_filter, meas_kind, d_mu, d_cov, cov_per_filter, d_mask);
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
-}
-
-/* ---- pipelined host-pointer calls -------------------------------------------------------------------------------- */
-static int pipe_make(ukfb_handle* h)
-{
-    if (h->pipe.made) return UKFB_OK;
-    CU(cudaStreamCreateWithFlags(&h->pipe.s_in, cudaStreamNonBlocking));
-    CU(cudaStreamCreateWithFlags(&h->pipe.s_out, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; ++i) {
-        CU(cudaEventCreateWithFlags(&h->pipe.in_ready[i], cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&h->pipe.in_consumed[i], cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&h->pipe.out_ready[i], cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&h->pipe.out_drained[i], cudaEventDisableTiming));
-    }
-    h->pipe.made = true;
-    return UKFB_OK;
-}
-
-static int pipe_reserve(ukfb_handle* h, char** buf, size_t* have, size_t bytes)
-{
-    if (bytes <= *have) return UKFB_OK;
-    CU(cudaStreamSynchronize(h->stream));
-    CU(cudaStreamSynchronize(h->pipe.s_in));
-    CU(cudaStreamSynchronize(h->pipe.s_out));
-    if (*buf) CU(cudaFree(*buf));
-    *buf = nullptr, *have = 0;
-    const size_t want = (bytes + (size_t(1) << 20)) & ~((size_t(1) << 20) - 1);
-    cudaError_t e = cudaMalloc(buf, want);
-    if (e != cudaSuccess) return fail(UKFB_ERR_NOMEM, "pipeline staging buffer of %zu bytes: %s", want, cudaGetErrorString(e));
-    *have = want;
-    return UKFB_OK;
+    return step_host(h, dt, dt_per_filter, meas_kind, mu, cov, cov_per_filter, mask, false, "ukfb_step");
 }
 
 /* ukfb_step without the final synchronisation: the inputs are copied on a copy-in stream into one of two staging
@@ -1622,106 +1714,7 @@ static int pipe_reserve(ukfb_handle* h, char** buf, size_t* have, size_t bytes)
 extern "C" int ukfb_step_async(ukfb_handle* h, const double* dt, int dt_per_filter, int meas_kind, const double* mu, const double* cov,
                                int cov_per_filter, const uint8_t* mask)
 {
-    CHECK_H(h);
-    NEED_INIT(h);
-    if (!dt) return fail(UKFB_ERR_INVALID, "ukfb_step_async: null dt");
-    const bool upd = meas_kind != UKFB_MEAS_NONE;
-    if (upd && !kind_ok(h, meas_kind)) return fail(UKFB_ERR_INVALID, "ukfb_step_async: measurement kind %d does not belong to this filter kind", meas_kind);
-    if (upd && !mu) return fail(UKFB_ERR_INVALID, "ukfb_step_async: null measurement");
-    if (upd && !cov && !h->meas_cov_per_filter[meas_kind]) return fail(UKFB_ERR_INVALID, "ukfb_step_async: null covariance and none kept by ukfb_set_measurement_cov for kind %d", meas_kind);
-    const int m = upd ? meas_dim(meas_kind) : 0;
-    UKFB_FAN(h, ukfb_step_async(s_, dt + (dt_per_filter ? f_ : 0), dt_per_filter, meas_kind, mu ? mu + f_ * m : nullptr,
-                                cov ? cov + (cov_per_filter ? f_ * m * m : 0) : nullptr, cov_per_filter, mask ? mask + f_ : nullptr));
-    int rc = pipe_make(h);
-    if (rc) return rc;
-    const int slot = int(h->pipe.n_in & 1);
-    const size_t bd = align256(sizeof(double) * (dt_per_filter ? h->B : 1));
-    const size_t bm = upd ? align256(sizeof(double) * h->B * m) : 0;
-    const size_t bc = (upd && cov) ? align256(sizeof(double) * (cov_per_filter ? h->B : 1) * m * m) : 0;
-    const size_t bk = (upd && mask) ? align256(size_t(h->B)) : 0;
-    rc = pipe_reserve(h, &h->pipe.in[slot], &h->pipe.in_bytes[slot], bd + bm + bc + bk);
-    if (rc) return rc;
-    char* base = h->pipe.in[slot];
-    cudaStream_t si = h->pipe.s_in;
-    if (h->pipe.n_in >= 2) CU(cudaStreamWaitEvent(si, h->pipe.in_consumed[slot], 0)); /* the kernel that read this slot is done */
-    CU(cudaMemcpyAsync(base, dt, sizeof(double) * (dt_per_filter ? h->B : 1), cudaMemcpyHostToDevice, si));
-    const double *d_mu = nullptr, *d_cov = nullptr;
-    const uint8_t* d_mask = nullptr;
-    if (upd) {
-        CU(cudaMemcpyAsync(base + bd, mu, sizeof(double) * h->B * m, cudaMemcpyHostToDevice, si));
-        d_mu = reinterpret_cast<const double*>(base + bd);
-        if (cov) {
-            CU(cudaMemcpyAsync(base + bd + bm, cov, sizeof(double) * (cov_per_filter ? h->B : 1) * m * m, cudaMemcpyHostToDevice, si));
-            d_cov = reinterpret_cast<const double*>(base + bd + bm);
-        } else
-            d_cov = h->meas_cov[meas_kind], cov_per_filter = h->meas_cov_per_filter[meas_kind] == 2;
-        if (mask) {
-            CU(cudaMemcpyAsync(base + bd + bm + bc, mask, size_t(h->B), cudaMemcpyHostToDevice, si));
-            d_mask = reinterpret_cast<const uint8_t*>(base + bd + bm + bc);
-        }
-    }
-    CU(cudaEventRecord(h->pipe.in_ready[slot], si));
-    CU(cudaStreamWaitEvent(h->stream, h->pipe.in_ready[slot], 0));
-    rc = ukfb_step_dev(h, reinterpret_cast<const double*>(base), dt_per_filter, meas_kind, d_mu, d_cov, cov_per_filter, d_mask);
-    if (rc) return rc;
-    CU(cudaEventRecord(h->pipe.in_consumed[slot], h->stream));
-    h->pipe.n_in++;
-    return UKFB_OK;
-}
-
-/* ukfb_get_state without the final synchronisation: the estimates of the steps issued so far are unpacked on the
- * compute stream into one of two staging slots and copied to the host on a copy-out stream, overlapping later
- * steps; mu / sigma are valid after ukfb_synchronize(). */
-extern "C" int ukfb_get_state_async(ukfb_handle* h, double* mu, double* sigma)
-{
-    CHECK_H(h);
-    NEED_INIT(h);
-    UKFB_FAN(h, ukfb_get_state_async(s_, mu ? mu + f_ * s_->MU : nullptr, sigma ? sigma + f_ * s_->n * s_->n : nullptr));
-    int rc = pipe_make(h);
-    if (rc) return rc;
-    const int slot = int(h->pipe.n_out & 1);
-    const size_t bm = align256(sizeof(double) * h->B * h->MU), bs = sizeof(double) * h->B * h->n * h->n;
-    rc = pipe_reserve(h, &h->pipe.out[slot], &h->pipe.out_bytes[slot], bm + (sigma ? bs : 0));
-    if (rc) return rc;
-    double* d_mu = reinterpret_cast<double*>(h->pipe.out[slot]);
-    double* d_sigma = reinterpret_cast<double*>(h->pipe.out[slot] + bm);
-    if (h->pipe.n_out >= 2) CU(cudaStreamWaitEvent(h->stream, h->pipe.out_drained[slot], 0)); /* the copy that read this slot is done */
-    rc = ukfb_get_state_dev(h, mu ? d_mu : nullptr, sigma ? d_sigma : nullptr);
-    if (rc) return rc;
-    CU(cudaEventRecord(h->pipe.out_ready[slot], h->stream));
-    cudaStream_t so = h->pipe.s_out;
-    CU(cudaStreamWaitEvent(so, h->pipe.out_ready[slot], 0));
-    if (mu) CU(cudaMemcpyAsync(mu, d_mu, sizeof(double) * h->B * h->MU, cudaMemcpyDeviceToHost, so));
-    if (sigma) CU(cudaMemcpyAsync(sigma, d_sigma, bs, cudaMemcpyDeviceToHost, so));
-    CU(cudaEventRecord(h->pipe.out_drained[slot], so));
-    h->pipe.n_out++;
-    return UKFB_OK;
-}
-
-extern "C" int ukfb_get_mu_range_async(ukfb_handle* h, int mu_first, int mu_count, double* out)
-{
-    CHECK_H(h);
-    NEED_INIT(h);
-    int rc = mu_range_ok(h, mu_first, mu_count, out, "ukfb_get_mu_range_async");
-    if (rc) return rc;
-    UKFB_FAN(h, ukfb_get_mu_range_async(s_, mu_first, mu_count, out + f_ * mu_count));
-    rc = pipe_make(h);
-    if (rc) return rc;
-    const int slot = int(h->pipe.n_out & 1);
-    const size_t bytes = sizeof(double) * h->B * mu_count;
-    rc = pipe_reserve(h, &h->pipe.out[slot], &h->pipe.out_bytes[slot], bytes);
-    if (rc) return rc;
-    double* d_out = reinterpret_cast<double*>(h->pipe.out[slot]);
-    if (h->pipe.n_out >= 2) CU(cudaStreamWaitEvent(h->stream, h->pipe.out_drained[slot], 0)); /* the copy that read this slot is done */
-    rc = ukfb_get_mu_range_dev(h, mu_first, mu_count, d_out);
-    if (rc) return rc;
-    CU(cudaEventRecord(h->pipe.out_ready[slot], h->stream));
-    cudaStream_t so = h->pipe.s_out;
-    CU(cudaStreamWaitEvent(so, h->pipe.out_ready[slot], 0));
-    CU(cudaMemcpyAsync(out, d_out, bytes, cudaMemcpyDeviceToHost, so));
-    CU(cudaEventRecord(h->pipe.out_drained[slot], so));
-    h->pipe.n_out++;
-    return UKFB_OK;
+    return step_host(h, dt, dt_per_filter, meas_kind, mu, cov, cov_per_filter, mask, true, "ukfb_step_async");
 }
 
 extern "C" int ukfb_run_dev(ukfb_handle* h, int K, const double* d_dt, int dt_per_filter, const int8_t* kinds_host, const double* d_mu3,
@@ -1814,14 +1807,6 @@ extern "C" int ukfb_run_events_dev(ukfb_handle* h, int K, const int64_t* d_ts_us
     return launch_step(h, p);
 }
 
-/* K rows of `cols` elements each, host -> device; the host rows are `src_cols` elements apart (a shard's slice of the
- * caller's slot-major K x B arrays), the device rows dense */
-static cudaError_t copy_rows_h2d(void* dst, const void* src, size_t elem, long long cols, long long src_cols, int rows, cudaStream_t st)
-{
-    if (cols == src_cols) return cudaMemcpyAsync(dst, src, elem * size_t(cols) * size_t(rows), cudaMemcpyHostToDevice, st);
-    return cudaMemcpy2DAsync(dst, elem * size_t(cols), src, elem * size_t(src_cols), elem * size_t(cols), size_t(rows), cudaMemcpyHostToDevice, st);
-}
-
 /* ukfb_run_events / ukfb_run_events_async on one device.  The arrays point at this handle's first filter in slot 0 and
  * their slots are src_B filters apart (src_B = h->B for a one-device handle, the parent's batch for a shard). */
 static int run_events_host(ukfb_handle* h, int K, const int64_t* ts_us, const int8_t* kinds, const double* mu3, const double* cov,
@@ -1829,48 +1814,21 @@ static int run_events_host(ukfb_handle* h, int K, const int64_t* ts_us, const in
 {
     CHECK_H(h);
     NEED_INIT(h);
-    const size_t n = size_t(K) * size_t(h->B);
-    const size_t bt = align256(sizeof(int64_t) * n), bk = align256(n), bm = align256(sizeof(double) * n * 3);
-    const size_t bc = sizeof(double) * (cov_mode ? n * 9 : size_t(UKFB_EVENT_KIND_COUNT) * 9);
-    char* base;
-    cudaStream_t si;
-    int slot = 0;
-    int rc;
-    if (async) {
-        rc = pipe_make(h);
-        if (rc) return rc;
-        slot = int(h->pipe.n_in & 1);
-        rc = pipe_reserve(h, &h->pipe.in[slot], &h->pipe.in_bytes[slot], bt + bk + bm + bc);
-        if (rc) return rc;
-        base = h->pipe.in[slot];
-        si = h->pipe.s_in;
-        if (h->pipe.n_in >= 2) CU(cudaStreamWaitEvent(si, h->pipe.in_consumed[slot], 0)); /* the launch that read this slot is done */
-    } else {
-        rc = stage_reserve(h, bt + bk + bm + bc);
-        if (rc) return rc;
-        base = h->stage;
-        si = h->stream;
-    }
-    CU(copy_rows_h2d(base, ts_us, sizeof(int64_t), h->B, src_B, K, si));
-    CU(copy_rows_h2d(base + bt, kinds, 1, h->B, src_B, K, si));
-    CU(copy_rows_h2d(base + bt + bk, mu3, sizeof(double) * 3, h->B, src_B, K, si));
+    const size_t B = size_t(h->B), pitch = size_t(src_B), rows = size_t(K);
+    const int64_t* d_ts;
+    const int8_t* d_kinds;
+    const double *d_mu3, *d_cov;
+    Staging st(h, async);
+    st.in_rows(&d_ts, ts_us, sizeof(int64_t) * B, rows, sizeof(int64_t) * pitch);
+    st.in_rows(&d_kinds, kinds, B, rows, pitch);
+    st.in_rows(&d_mu3, mu3, sizeof(double) * 3 * B, rows, sizeof(double) * 3 * pitch);
     if (cov_mode)
-        CU(copy_rows_h2d(base + bt + bk + bm, cov, sizeof(double) * 9, h->B, src_B, K, si));
+        st.in_rows(&d_cov, cov, sizeof(double) * 9 * B, rows, sizeof(double) * 9 * pitch);
     else
-        CU(cudaMemcpyAsync(base + bt + bk + bm, cov, bc, cudaMemcpyHostToDevice, si));
-    if (async) {
-        CU(cudaEventRecord(h->pipe.in_ready[slot], si));
-        CU(cudaStreamWaitEvent(h->stream, h->pipe.in_ready[slot], 0));
-    }
-    rc = ukfb_run_events_dev(h, K, reinterpret_cast<const int64_t*>(base), reinterpret_cast<const int8_t*>(base + bt),
-                             reinterpret_cast<const double*>(base + bt + bk), reinterpret_cast<const double*>(base + bt + bk + bm), cov_mode);
-    if (rc) return rc;
-    if (async) {
-        CU(cudaEventRecord(h->pipe.in_consumed[slot], h->stream));
-        h->pipe.n_in++;
-    } else
-        CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+        st.in(&d_cov, cov, sizeof(double) * UKFB_EVENT_KIND_COUNT * 9);
+    int rc = st.commit();
+    if (!rc) rc = ukfb_run_events_dev(h, K, d_ts, d_kinds, d_mu3, d_cov, cov_mode);
+    return rc ? rc : st.finish();
 }
 
 static int run_events_any(ukfb_handle* h, int K, const int64_t* ts_us, const int8_t* kinds, const double* mu3, const double* cov,
@@ -2060,19 +2018,15 @@ static int get_state_indexed_one(ukfb_handle* h, int64_t n, const int64_t* idx, 
 {
     CHECK_H(h); /* a shard runs this on its worker thread: select its device there */
     if (n == 0) return UKFB_OK;
-    const size_t bi = align256(sizeof(int64_t) * n), bm = align256(sizeof(double) * n * h->MU), bs = sizeof(double) * n * h->n * h->n;
-    int rc = stage_reserve(h, bi + bm + (sigma ? bs : 0));
-    if (rc) return rc;
-    long long* d_idx = reinterpret_cast<long long*>(h->stage);
-    double* d_mu = reinterpret_cast<double*>(h->stage + bi);
-    double* d_sigma = reinterpret_cast<double*>(h->stage + bi + bm);
-    CU(cudaMemcpyAsync(d_idx, idx, sizeof(int64_t) * n, cudaMemcpyHostToDevice, h->stream));
-    rc = get_state_indexed_launch(h, n, d_idx, d_mu, sigma ? d_sigma : nullptr);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(mu, d_mu, sizeof(double) * n * h->MU, cudaMemcpyDeviceToHost, h->stream));
-    if (sigma) CU(cudaMemcpyAsync(sigma, d_sigma, bs, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    const long long* d_idx;
+    double *d_mu, *d_sigma;
+    Staging st(h, false);
+    st.in(&d_idx, idx, sizeof(int64_t) * n);
+    st.out(&d_mu, mu, sizeof(double) * n * h->MU);
+    st.out(&d_sigma, sigma, sizeof(double) * n * h->n * h->n);
+    int rc = st.commit();
+    if (!rc) rc = get_state_indexed_launch(h, n, d_idx, d_mu, d_sigma);
+    return rc ? rc : st.finish();
 }
 
 extern "C" int ukfb_get_state_indexed(ukfb_handle* h, int64_t n, const int64_t* idx, double* mu, double* sigma)
@@ -2134,19 +2088,15 @@ static int initialize_indexed_one(ukfb_handle* h, int64_t n, const int64_t* idx,
 {
     CHECK_H(h); /* a shard runs this on its worker thread: select its device there */
     if (n == 0) return UKFB_OK;
-    const size_t bi = align256(sizeof(int64_t) * n), bm = align256(sizeof(double) * n * h->MU), bs = sizeof(double) * n * h->n * h->n;
-    int rc = stage_reserve(h, bi + bm + bs);
-    if (rc) return rc;
-    long long* d_idx = reinterpret_cast<long long*>(h->stage);
-    double* d_mu = reinterpret_cast<double*>(h->stage + bi);
-    double* d_sigma = reinterpret_cast<double*>(h->stage + bi + bm);
-    CU(cudaMemcpyAsync(d_idx, idx, sizeof(int64_t) * n, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(d_mu, mu, sizeof(double) * n * h->MU, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(d_sigma, sigma, bs, cudaMemcpyHostToDevice, h->stream));
-    rc = initialize_indexed_launch(h, n, d_idx, d_mu, d_sigma);
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    const long long* d_idx;
+    const double *d_mu, *d_sigma;
+    Staging st(h, false);
+    st.in(&d_idx, idx, sizeof(int64_t) * n);
+    st.in(&d_mu, mu, sizeof(double) * n * h->MU);
+    st.in(&d_sigma, sigma, sizeof(double) * n * h->n * h->n);
+    int rc = st.commit();
+    if (!rc) rc = initialize_indexed_launch(h, n, d_idx, d_mu, d_sigma);
+    return rc ? rc : st.finish();
 }
 
 extern "C" int ukfb_initialize_indexed(ukfb_handle* h, int64_t n, const int64_t* idx, const double* mu, const double* sigma)
@@ -2189,7 +2139,7 @@ static int find_status_one(ukfb_handle* h, uint32_t bits, int64_t max_n, int64_t
     const long long chunks = (h->B + FS_CHUNK - 1) / FS_CHUNK;
     const long long cap = max_n < h->B ? (long long)max_n : h->B;
     const size_t bc = align256(sizeof(long long) * (chunks + 1));
-    int rc = stage_reserve(h, bc + sizeof(long long) * (cap > 0 ? cap : 1));
+    int rc = stage_grow(h, h->stage, h->stage_bytes, bc + sizeof(long long) * (cap > 0 ? cap : 1), false);
     if (rc) return rc;
     IndexParams p = index_params(h, chunks, nullptr);
     p.bits = bits;
@@ -2246,14 +2196,14 @@ static int clear_status_indexed_one(ukfb_handle* h, int64_t n, const int64_t* id
 {
     CHECK_H(h); /* a shard runs this on its worker thread: select its device there */
     if (n == 0) return UKFB_OK;
-    int rc = stage_reserve(h, sizeof(int64_t) * n);
+    const long long* d_idx;
+    Staging st(h, false);
+    st.in(&d_idx, idx, sizeof(int64_t) * n);
+    int rc = st.commit();
     if (rc) return rc;
-    long long* d_idx = reinterpret_cast<long long*>(h->stage);
-    CU(cudaMemcpyAsync(d_idx, idx, sizeof(int64_t) * n, cudaMemcpyHostToDevice, h->stream));
     clear_status_indexed_kernel<<<grid_for(n), 256, 0, h->stream>>>(index_params(h, n, d_idx));
     CU(cudaGetLastError());
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    return st.finish();
 }
 
 extern "C" int ukfb_clear_status_indexed(ukfb_handle* h, int64_t n, const int64_t* idx)
@@ -2394,17 +2344,17 @@ extern "C" int ukfb_selftest_so3(ukfb_handle* h, int64_t n, const double* v, con
     CHECK_H(h);
     if (n < 1 || !v || !x || !out) return fail(UKFB_ERR_INVALID, "ukfb_selftest_so3: bad argument");
     if (is_sharded(h)) return ukfb_selftest_so3(h->shards[0], n, v, x, out);
-    const size_t bv = align256(sizeof(double) * n * 3), bx = align256(sizeof(double) * n), bo = sizeof(double) * n * UKFB_SELFTEST_STRIDE;
-    int rc = stage_reserve(h, bv + bx + bo);
+    const double *d_v, *d_x;
+    double* d_out;
+    Staging st(h, false);
+    st.in(&d_v, v, sizeof(double) * n * 3);
+    st.in(&d_x, x, sizeof(double) * n);
+    st.out(&d_out, out, sizeof(double) * n * UKFB_SELFTEST_STRIDE);
+    int rc = st.commit();
     if (rc) return rc;
-    CU(cudaMemcpyAsync(h->stage, v, sizeof(double) * n * 3, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(h->stage + bv, x, sizeof(double) * n, cudaMemcpyHostToDevice, h->stream));
-    so3_selftest_kernel<<<grid_for(n), 256, 0, h->stream>>>(reinterpret_cast<const double*>(h->stage), reinterpret_cast<const double*>(h->stage + bv),
-                                                            reinterpret_cast<double*>(h->stage + bv + bx), n);
+    so3_selftest_kernel<<<grid_for(n), 256, 0, h->stream>>>(d_v, d_x, d_out, n);
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(out, h->stage + bv + bx, bo, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    return UKFB_OK;
+    return st.finish();
 }
 
 extern "C" int ukfb_measure_fp64_peak(ukfb_handle* h, double* flops_per_s)
@@ -2412,7 +2362,7 @@ extern "C" int ukfb_measure_fp64_peak(ukfb_handle* h, double* flops_per_s)
     CHECK_H(h);
     if (!flops_per_s) return fail(UKFB_ERR_INVALID, "ukfb_measure_fp64_peak: null argument");
     if (is_sharded(h)) return ukfb_measure_fp64_peak(h->shards[0], flops_per_s);
-    int rc = stage_reserve(h, 256);
+    int rc = stage_grow(h, h->stage, h->stage_bytes, 256, false);
     if (rc) return rc;
     cudaDeviceProp prop;
     CU(cudaGetDeviceProperties(&prop, h->device));

@@ -596,6 +596,70 @@ def test_streaming_calls_match_the_blocking_ones(Ukf):
     assert np.array_equal(a.get_state()[0], b.get_state()[0])
 
 
+@pytest.mark.parametrize("devices", [None, [0, 0, 0]])
+def test_streaming_calls_match_the_blocking_ones_over_every_staged_layout(Ukf, devices):
+    """step_async / get_state_async / get_mu_range_async against their blocking twins on a second handle, bit for bit,
+    over every set of arrays a call stages: dt broadcast or per filter; no measurement, a broadcast R, a per-filter R or
+    the R kept by set_measurement_cov (cov=None); with and without a mask; mu alone, mu and sigma, or a range of mu.
+    36 000 filters, 12 000 per shard on three: the third step lands in the input slot of the first (dt alone, 1 MiB) and
+    needs more (97 bytes per filter with a per-filter R and a mask), the third read-back (sigma) in the output slot of
+    the first (a range of mu), so both slots grow between pipelined calls."""
+    import torch
+
+    B = 36000
+    rng = np.random.default_rng(11)
+    keep = []
+
+    def pinned(x):
+        t = torch.from_numpy(np.ascontiguousarray(x)).pin_memory()
+        keep.append(t)
+        return t.numpy()
+
+    a, b = P.make_pose(Ukf, B), P.make_pose(Ukf, B, devices=devices)
+    kept_R = syn.pose_measurement(0, B, 1)[1] * rng.uniform(0.5, 2.0, (B, 1, 1))
+    for x in (a, b):
+        x.set_measurement_cov(0, kept_R)
+    # (dt per filter, measurement, mask): the 14 combinations, starting with the ones that make the slots grow
+    seq = [(False, "none", False), (True, "per", True), (False, "per", True), (True, "bcast", False), (False, "kept", True),
+           (True, "none", False), (False, "bcast", True), (True, "kept", False), (False, "per", False), (True, "bcast", True),
+           (False, "kept", False), (True, "per", False), (True, "kept", True), (False, "bcast", False)]
+    assert len(set(seq)) == 14
+    want, got = [], []
+    for k, (dt_per, meas, masked) in enumerate(seq):
+        dt = pinned(syn.DT * rng.uniform(0.5, 1.5, B)) if dt_per else syn.DT
+        kind, mu, cov = -1, None, None
+        if meas == "bcast":
+            kind = 8
+            mu, cov = syn.pose_measurement(kind, B, k + 1)
+        elif meas == "per":
+            kind = 4
+            mu, R = syn.pose_measurement(kind, B, k + 1)
+            cov = pinned(R * rng.uniform(0.5, 2.0, (B, 1, 1)))
+        elif meas == "kept":
+            kind = 0
+            mu = syn.pose_measurement(kind, B, k + 1)[0]
+        mu = pinned(mu) if mu is not None else None
+        mask = pinned(rng.integers(0, 2, B, dtype=np.uint8)) if masked else None
+        a.step(dt, kind, mu, cov, mask)
+        b.step_async(dt, kind, mu, cov, mask)
+        if k % 3 == 0:
+            want.append((a.get_mu_range(0, 7),))
+            got.append((pinned(np.empty((B, 7))),))
+            b.get_mu_range_async(0, 7, *got[-1])
+        elif k % 3 == 1:
+            want.append((a.get_state(with_sigma=False),))
+            got.append((pinned(np.empty((B, 13))),))
+            b.get_state_async(*got[-1])
+        else:
+            want.append(a.get_state())
+            got.append((pinned(np.empty((B, 13))), pinned(np.empty((B, 12, 12)))))
+            b.get_state_async(*got[-1])
+    b.synchronize()
+    for k, (w, g) in enumerate(zip(want, got)):
+        for wi, gi in zip(w, g):
+            assert np.array_equal(gi, wi), f"step {k} {seq[k]}: streamed read-back differs from the blocking one"
+
+
 @pytest.mark.gpu
 def test_fast_kernel_not_spd_deferral_is_one_factorisation():
     """see tests/test_emu_lane_kernels.py::check_not_spd_deferral: the documented one-step deferral, on the device"""
