@@ -116,6 +116,20 @@ public:
      * initializeFilter(index, ...); empty after a call that threw nothing */
     const std::vector<int64_t>& lastFailedFilters() const { return failed; }
 
+    /* One image of the whole object (include/ukf_batch.h, "checkpoint / restore"): every filter's state, covariance, time
+     * latch, status, stored samples, process noise and the object-wide settings.  restoreCheckpoint brings an object of
+     * the same filter kind and batch size -- on any number of GPUs -- back exactly to the saved point; a rejected image
+     * throws as every failed call does and leaves the object unchanged. */
+    std::vector<uint8_t> saveCheckpoint() const
+    {
+        uint64_t bytes = 0;
+        check(ukfb_checkpoint_size(h, &bytes));
+        std::vector<uint8_t> image(static_cast<size_t>(bytes));
+        check(ukfb_checkpoint_save(h, image.data(), bytes));
+        return image;
+    }
+    void restoreCheckpoint(const std::vector<uint8_t>& image) { check(ukfb_checkpoint_restore(h, image.data(), image.size())); }
+
     /* :83-100; sample_time in microseconds (base::Time::microseconds) */
     void predictionStepFromSampleTime(int64_t sample_time_us)
     {

@@ -340,6 +340,74 @@ int ukfb_find_status(ukfb_handle* h, uint32_t bits, int64_t max_n, int64_t* idx,
 /* status words of filters idx[0..n) set to 0 (ukfb_clear_status for a subset); duplicates allowed */
 int ukfb_clear_status_indexed(ukfb_handle* h, int64_t n, const int64_t* idx);
 
+/* ---- checkpoint / restore ---------------------------------------------------------------------------------------- */
+/* One image of everything a batch holds for its filters, so that a stopped job resumes exactly where it stopped, on the
+ * same or another number of devices and with any kernel family (UKFB_KERNEL):  records (mu, sigma), t_last, status
+ * words, the stored acceleration / IMU sample, Q, per-filter orientation parameters, kept measurement covariances, and
+ * the handle-wide values (time bounds, gate, orientation parameters, mean-pass histogram, initialized / first-init).
+ * Launch configuration, pipeline slots, launch counters and the launch-overlap counters are not filter state and are
+ * not saved.
+ *
+ * Image: a flat little-endian byte buffer, a 768-byte header, then one section per array.
+ *   header    offset  type         field
+ *             0       char[8]      magic "UKFBCKPT"
+ *             8       uint32       version (UKFB_CHECKPOINT_VERSION)
+ *             12      uint32       header bytes (768)
+ *             16      uint64       total bytes of the image
+ *             24      int32 x 3    kind, MU, n
+ *             36      uint32       number of section-table entries (UKFB_CKPT_SECTIONS)
+ *             40      int64        B
+ *             48      uint32 x 2   initialized, first_init (0 / 1)
+ *             56      double x 2   min_dt, max_dt
+ *             72      double       Mahalanobis gate
+ *             80      double x 6   tau_g, tau_a, latitude, earth[3] (the handle-wide orientation parameters)
+ *             128     uint64 x 8   mean-pass histogram (ukfb_get_mean_iter_hist: summed over the handle's slots and shards)
+ *             192     uint32 x 2   Q per filter (0 / 1), per-filter orientation parameters present (0 / 1)
+ *             200     uint32 x 10  kept covariance of measurement kind k (ukfb_set_measurement_cov): 0 none,
+ *                                  1 broadcast, 2 per filter
+ *             240     16 zero bytes
+ *             256     18 x 24      section table, entry i for section id i: uint32 id, uint32 0, uint64 offset,
+ *                                  uint64 bytes; an absent section has offset 0 and bytes 0
+ *   sections, at 256-byte aligned offsets in id order, filter-major, all B filters in global filter order:
+ *     id 0        records       REC doubles per filter: mu, then the packed lower triangle of sigma (tri(r, c) order)
+ *     id 1        t_last        int64
+ *     id 2        status        uint32
+ *     id 3, 4, 5  acc_mu (3), acc_cov (9), gyro_mu (3) doubles: the stored samples, NaN sentinel of PoseUKF included
+ *     id 6        Q             the packed lower triangle (n (n + 1) / 2 doubles) per filter, or once when broadcast
+ *     id 7        orientation parameters, 5 doubles per filter (-1/tau_g, -1/tau_a, earth xyz as stored); only if present
+ *     id 8 + k    kept covariance of measurement kind k, m x m per filter, or once when broadcast; only if kept
+ * The bytes of an image depend on the filters' state alone: not on the shard count, nor on the kernel family.  Per filter:
+ * 860 bytes (PoseUKF) / 972 (OrientationUKF), + 624 / 728 with per-filter Q, + 40 with per-filter orientation parameters.
+ *
+ *   ukfb_checkpoint_size: bytes of this handle's image now (the modes above decide it).
+ *   ukfb_checkpoint_save: UKFB_ERR_NOT_INITIALIZED on a handle never initialized; UKFB_ERR_INVALID for a null buffer or
+ *     one smaller than ukfb_checkpoint_size.
+ *   ukfb_checkpoint_restore: checks magic, version, kind, B, MU, n, every section's offset and size against the header's
+ *     modes, and that the image fits `bytes`, before anything is enqueued on any shard: a rejected image (UKFB_ERR_INVALID)
+ *     leaves the handle unchanged.  Then replaces every per-filter and handle-wide value above, reallocating Q, the
+ *     orientation parameters and kept covariances whose mode differs, as the setters do; initialized / first_init come
+ *     from the image (a later ukfb_initialize of a restored OrientationUKF handle does not apply the constructor's
+ *     defaults again).  On a sharded handle shard i reads / writes rows [first_i, first_i + count_i) of every section;
+ *     handle-wide values are saved from shard 0; a restored histogram goes to shard 0 whole.  An image of any shard
+ *     count restores onto any other.
+ *   `_dev` variants: the image in device memory of the handle's device (UKFB_ERR_INVALID on a sharded parent).  The save
+ *     only enqueues; the restore reads the header (with a broadcast Q behind it) back in one small synchronous copy to
+ *     validate it, the payload stays on the device: an in-device snapshot and rollback.
+ *   Host-pointer calls move the record section through a device buffer of at most 64 MiB (kept by the handle, as every
+ *   staging buffer); the other sections go straight between the caller's buffer and the handle's arrays.  A restore
+ *   allocates every array whose size changes before it frees the old one: UKFB_ERR_NOMEM leaves a one-device handle as it
+ *   was; on a sharded handle it names the shard that failed, the other shards are restored.
+ * All work is plain launches and cudaMemcpyAsync on the handle's stream, in full stream order with earlier _async calls
+ * and with step launches that overlap one another tile by tile. */
+#define UKFB_CHECKPOINT_VERSION 1
+#define UKFB_CKPT_HEADER_BYTES 768
+#define UKFB_CKPT_SECTIONS 18
+int ukfb_checkpoint_size(ukfb_handle* h, uint64_t* bytes);
+int ukfb_checkpoint_save(ukfb_handle* h, void* buf, uint64_t bytes);
+int ukfb_checkpoint_restore(ukfb_handle* h, const void* buf, uint64_t bytes);
+int ukfb_checkpoint_save_dev(ukfb_handle* h, void* d_buf, uint64_t bytes);
+int ukfb_checkpoint_restore_dev(ukfb_handle* h, const void* d_buf, uint64_t bytes);
+
 /* ---- stream plumbing ------------------------------------------------------- */
 
 int ukfb_synchronize(ukfb_handle* h);

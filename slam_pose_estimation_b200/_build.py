@@ -14,8 +14,9 @@ CSRC = os.path.join(_PKG, "csrc")
 # UKFB_LIB: load another build of the same library (kernel tuning experiments)
 LIB = os.environ.get("UKFB_LIB") or os.path.join(_PKG, "lib", "libukfb.so")
 SOURCES = ["ukf_batch.cu"]
-DEPS = ["ukf_batch.cu", "ukf_device.cuh", "ukf_thread.cuh", "ukf_pose_fast.cuh", "ukf_ori_fast.cuh", "ukf_index.cuh", "so3.cuh", "simt.cuh", "../../include/ukf_batch.h", "../../include/ukfb_constants.h"]
-# the step kernels' sources: what source_hash() covers (ukf_index.cuh holds per-filter access kernels, no step code)
+DEPS = ["ukf_batch.cu", "ukf_device.cuh", "ukf_thread.cuh", "ukf_pose_fast.cuh", "ukf_ori_fast.cuh", "ukf_index.cuh", "ukf_checkpoint.cuh", "so3.cuh", "simt.cuh", "../../include/ukf_batch.h", "../../include/ukfb_constants.h"]
+# the step kernels' sources: what source_hash() covers (ukf_index.cuh and ukf_checkpoint.cuh hold per-filter access and
+# checkpoint kernels, no step code)
 STEP_KERNEL_SOURCES = ["simt.cuh", "so3.cuh", "ukf_device.cuh", "ukf_ori_fast.cuh", "ukf_pose_fast.cuh", "ukf_thread.cuh"]
 
 NVCC_FLAGS = [

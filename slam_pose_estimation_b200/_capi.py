@@ -84,6 +84,11 @@ SIGNATURES = {
     "ukfb_initialize_indexed_dev": (I, [P, L, P, P, P]),
     "ukfb_find_status": (I, [P, C.c_uint32, L, P, C.POINTER(L)]),
     "ukfb_clear_status_indexed": (I, [P, L, P]),
+    "ukfb_checkpoint_size": (I, [P, C.POINTER(C.c_uint64)]),
+    "ukfb_checkpoint_save": (I, [P, P, C.c_uint64]),
+    "ukfb_checkpoint_restore": (I, [P, P, C.c_uint64]),
+    "ukfb_checkpoint_save_dev": (I, [P, P, C.c_uint64]),
+    "ukfb_checkpoint_restore_dev": (I, [P, P, C.c_uint64]),
     "ukfb_synchronize": (I, [P]),
     "ukfb_stream": (P, [P]),
     "ukfb_event_record": (I, [P, I]),

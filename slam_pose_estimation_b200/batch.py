@@ -498,6 +498,67 @@ class UkfBatch:
         idx, pi = _index_array(idx, "clear_status_indexed")
         self._chk(self.lib.ukfb_clear_status_indexed(self.h, idx.size, pi))
 
+    # ---- checkpoint / restore (image format: include/ukf_batch.h) ----------------------------------------
+    def checkpoint_size(self) -> int:
+        """bytes of this batch's checkpoint image now (Q, orientation-parameter and kept-covariance modes decide it)"""
+        n = C.c_uint64()
+        self._chk(self.lib.ukfb_checkpoint_size(self.h, C.byref(n)))
+        return n.value
+
+    def checkpoint(self, out: np.ndarray | None = None) -> np.ndarray:
+        """one image of every filter's full state and the batch's handle-wide values, as a np.uint8 array (into `out`, a
+        uint8 array of at least checkpoint_size() bytes -- pinned for speed -- if given).  Writing it to disk is
+        `img.tofile(path)`; it restores onto a batch of the same kind and size on any number of devices."""
+        size = self.checkpoint_size()
+        if out is None:
+            out = np.empty(size, np.uint8)
+        elif out.dtype != np.uint8 or not out.flags.c_contiguous or out.size < size:
+            raise ValueError(f"checkpoint: out must be a contiguous uint8 array of at least {size} bytes")
+        self._chk(self.lib.ukfb_checkpoint_save(self.h, out.ctypes.data_as(C.c_void_p), out.size))
+        return out[:size]
+
+    def restore(self, buf):
+        """replace this batch's whole state by an image of checkpoint(): bytes, bytearray or a uint8 array.  A rejected
+        image (other kind or size, bad version, truncated) raises UkfbError and changes nothing."""
+        if isinstance(buf, (bytes, bytearray, memoryview)):
+            a = np.frombuffer(buf, np.uint8)
+        else:
+            a = np.asarray(buf)
+            if a.dtype != np.uint8:
+                raise TypeError(f"restore: the image must be bytes, bytearray or a uint8 array, got {a.dtype}")
+            a = np.ascontiguousarray(a.reshape(-1))
+        self._chk(self.lib.ukfb_checkpoint_restore(self.h, a.ctypes.data_as(C.c_void_p), a.size))
+
+    def checkpoint_dev(self, out=None):
+        """the image into a CUDA torch.uint8 tensor on this batch's device (allocated if None), enqueued on the handle's
+        stream and ordered before later work of the torch stream: an in-device snapshot for rollback (restore_dev)"""
+        import torch
+
+        size = self.checkpoint_size()
+        if out is None:
+            out = torch.empty(size, dtype=torch.uint8, device=f"cuda:{self.device}")
+        elif out.dtype != torch.uint8 or not out.is_cuda or out.numel() < size or not out.is_contiguous():
+            raise ValueError(f"checkpoint_dev: out must be a contiguous CUDA uint8 tensor of at least {size} bytes")
+        elif out.device.index != self.device:
+            raise ValueError(f"checkpoint_dev: out is on {out.device}, this batch on cuda:{self.device}")
+        self._after_torch(out)  # torch may still be using the buffer
+        self._chk(self.lib.ukfb_checkpoint_save_dev(self.h, _dev(out), out.numel()))
+        self._before_torch(out)
+        return out
+
+    def restore_dev(self, t):
+        """replace this batch's state by an image in a CUDA torch.uint8 tensor (checkpoint_dev); the header is read back
+        to be checked, the payload stays on the device"""
+        import torch
+
+        if t.dtype != torch.uint8 or not t.is_cuda:
+            raise ValueError("restore_dev: the image must be a CUDA uint8 tensor")
+        if t.device.index != self.device:
+            raise ValueError(f"restore_dev: the image is on {t.device}, this batch on cuda:{self.device}")
+        self._after_torch(t)
+        self._chk(self.lib.ukfb_checkpoint_restore_dev(self.h, _dev(t), t.numel()))
+        self._before_torch(t)  # torch must not overwrite the image before it has been read
+
     # ---- stream plumbing ------------------------------------------------------------------------------
     def synchronize(self):
         self._chk(self.lib.ukfb_synchronize(self.h))

@@ -11,12 +11,14 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <array>
 #include <cassert>
 #include <cfloat>
 #include <cmath>
 #include <vector>
 #include <cstdarg>
 #include <cstdio>
+#include <cstddef>
 #include <cstring>
 #include <new>
 #include <condition_variable>
@@ -29,6 +31,7 @@
 #include "ukf_device.cuh"
 #include "ukf_thread.cuh"
 #include "ukf_index.cuh"
+#include "ukf_checkpoint.cuh"
 #ifndef UKFB_DEFAULT_PREFETCH_BYTES
 #define UKFB_DEFAULT_PREFETCH_BYTES 128
 #endif
@@ -190,6 +193,10 @@ struct Staging {
     void in_rows(T** dev, const void* src, size_t width, size_t rows, size_t pitch) { add(dev, src, nullptr, width, rows, pitch); }
     template <class T>
     void out(T** dev, void* dst, size_t bytes) { add(dev, nullptr, dst, bytes, 1, bytes); }
+    /* device room without copies: the call moves the data itself, on h->stream (the checkpoint calls, whose sections go
+     * to or come from several places of the caller's buffer) */
+    template <class T>
+    void scratch(T** dev, size_t bytes) { add(dev, nullptr, nullptr, bytes, 1, bytes, true); }
 
     int commit()
     {
@@ -264,10 +271,10 @@ private:
         char* at;                 /* device address, from commit() on */
     };
     template <class T>
-    void add(T** dev, const void* src, void* dst, size_t width, size_t rows, size_t pitch)
+    void add(T** dev, const void* src, void* dst, size_t width, size_t rows, size_t pitch, bool keep = false)
     {
         *dev = nullptr;
-        if (!src && !dst) return;
+        if (!src && !dst && !keep) return;
         assert(n < MAX_PARTS);
         part[n++] = Part{dev, [](void* d, char* a) { *static_cast<T**>(d) = reinterpret_cast<T*>(a); }, src, dst, width, rows, pitch, nullptr};
     }
@@ -646,6 +653,7 @@ struct EnvKnobs {
     bool overlap;              /* UKFB_OVERLAP_LAUNCHES=0: every fast-kernel launch waits for the whole previous one */
     int overlap_max_waves;     /* UKFB_OVERLAP_MAX_WAVES: overlap launches of grids up to this many waves of resident warps (12) */
     int overlap_min_waves_pct; /* UKFB_OVERLAP_MIN_WAVES_PCT: ... and of more than this many hundredths of a wave (100) */
+    bool ckpt_elem;            /* UKFB_CKPT_TRANSFORM=elem: checkpoint record transforms per element instead of per tile */
     EnvKnobs()
     {
         const char* e = getenv("UKFB_FAST_WPB");
@@ -663,6 +671,8 @@ struct EnvKnobs {
         overlap_max_waves = e && atoi(e) > 0 ? atoi(e) : 12;
         e = getenv("UKFB_OVERLAP_MIN_WAVES_PCT");
         overlap_min_waves_pct = e ? atoi(e) : 100;
+        e = getenv("UKFB_CKPT_TRANSFORM");
+        ckpt_elem = e && strcmp(e, "elem") == 0;
     }
 };
 static const EnvKnobs& knobs()
@@ -1241,6 +1251,18 @@ extern "C" int ukfb_get_mu_range_async(ukfb_handle* h, int mu_first, int mu_coun
     return get_mu_range_host(h, mu_first, mu_count, out, true, "ukfb_get_mu_range_async");
 }
 
+/* StepParams::q_diagonal of a broadcast Q, from its packed lower triangle: 1 = no off-diagonal entry, 2 = that and one
+ * value on the diagonal of each of the first two 3 x 3 blocks, 0 = neither.  ukfb_set_process_noise and the checkpoint
+ * restore both classify with this, so that a restored handle takes the step kernels' path the saved one took. */
+static int broadcast_q_class(const double* Qp, int n)
+{
+    for (int r = 0; r < n; ++r)
+        for (int c = 0; c < r; ++c)
+            if (Qp[tri(r, c)] != 0.0) return 0;
+    const double a = Qp[tri(0, 0)], b = Qp[tri(3, 3)];
+    return a == Qp[tri(1, 1)] && a == Qp[tri(2, 2)] && b == Qp[tri(4, 4)] && b == Qp[tri(5, 5)] ? 2 : 1;
+}
+
 extern "C" int ukfb_set_process_noise(ukfb_handle* h, const double* Q, int per_filter)
 {
     CHECK_H(h);
@@ -1263,13 +1285,10 @@ extern "C" int ukfb_set_process_noise(ukfb_handle* h, const double* Q, int per_f
     }
     h->q_diagonal = 0;
     if (!per_filter) { /* the lower triangle is what pack_q_kernel keeps */
-        h->q_diagonal = 1;
+        double qp[OriF::LP];
         for (int r = 0; r < h->n; ++r)
-            for (int c = 0; c < r; ++c)
-                if (Q[r * h->n + c] != 0.0) h->q_diagonal = 0;
-        const int n = h->n;
-        if (h->q_diagonal && Q[0] == Q[n + 1] && Q[0] == Q[2 * n + 2] && Q[3 * n + 3] == Q[4 * n + 4] && Q[3 * n + 3] == Q[5 * n + 5])
-            h->q_diagonal = 2;
+            for (int c = 0; c <= r; ++c) qp[tri(r, c)] = Q[r * h->n + c];
+        h->q_diagonal = broadcast_q_class(qp, h->n);
     }
     pack_q_kernel<<<grid_for(count * h->LP), 256, 0, h->stream>>>(h->Q, d_Q, count, h->n, h->LP);
     CU(cudaGetLastError());
@@ -2223,6 +2242,466 @@ extern "C" int ukfb_clear_status_indexed(ukfb_handle* h, int64_t n, const int64_
     } catch (const std::bad_alloc&) {
         return fail(UKFB_ERR_NOMEM, "ukfb_clear_status_indexed: out of host memory");
     }
+}
+
+/* ---- checkpoint / restore (format: include/ukf_batch.h; record transforms: ukf_checkpoint.cuh) ----------------------- */
+enum { CK_RECORDS, CK_T_LAST, CK_STATUS, CK_ACC_MU, CK_ACC_COV, CK_GYRO_MU, CK_Q, CK_ORI, CK_MEAS0 };
+static_assert(CK_MEAS0 + UKFB_MEAS_KIND_COUNT == UKFB_CKPT_SECTIONS, "one section per measurement kind");
+
+struct CkptSection {
+    uint32_t id, zero;
+    uint64_t offset, bytes;
+};
+struct CkptHeader {
+    char magic[8];
+    uint32_t version, header_bytes;
+    uint64_t total_bytes;
+    int32_t kind, MU, n;
+    uint32_t n_sections;
+    int64_t B;
+    uint32_t initialized, first_init;
+    double min_dt, max_dt, gate_d2, tau_g, tau_a, latitude, earth[3];
+    uint64_t hist[8];
+    uint32_t q_per_filter, has_ori_params;
+    uint32_t meas_cov_mode[UKFB_MEAS_KIND_COUNT]; /* 0 none, 1 broadcast, 2 per filter: ukfb_handle::meas_cov_per_filter */
+    uint8_t zero[16];
+    CkptSection section[UKFB_CKPT_SECTIONS];
+    uint8_t pad[UKFB_CKPT_HEADER_BYTES - 256 - UKFB_CKPT_SECTIONS * sizeof(CkptSection)];
+};
+static_assert(sizeof(CkptHeader) == UKFB_CKPT_HEADER_BYTES && offsetof(CkptHeader, B) == 40 && offsetof(CkptHeader, min_dt) == 56 &&
+                  offsetof(CkptHeader, hist) == 128 && offsetof(CkptHeader, q_per_filter) == 192 &&
+                  offsetof(CkptHeader, meas_cov_mode) == 200 && offsetof(CkptHeader, section) == 256,
+              "the header layout of include/ukf_batch.h");
+static const char CKPT_MAGIC[8] = {'U', 'K', 'F', 'B', 'C', 'K', 'P', 'T'};
+
+/* what decides the sections an image has */
+struct CkptModes {
+    uint32_t q_per_filter = 0, has_ori_params = 0;
+    uint32_t meas[UKFB_MEAS_KIND_COUNT] = {};
+};
+
+static CkptModes ckpt_modes(const ukfb_handle* h) /* a one-device handle: its own; a sharded parent: shard 0's (the setters fan out) */
+{
+    const ukfb_handle* s = is_sharded(h) ? h->shards[0] : h;
+    CkptModes m;
+    m.q_per_filter = s->q_per_filter ? 1 : 0;
+    m.has_ori_params = s->ori_params ? 1 : 0;
+    for (int k = 0; k < UKFB_MEAS_KIND_COUNT; ++k) m.meas[k] = uint32_t(s->meas_cov_per_filter[k]);
+    return m;
+}
+
+/* where the sections of an image of B filters lie */
+struct CkptLayout {
+    uint64_t off[UKFB_CKPT_SECTIONS] = {}, bytes[UKFB_CKPT_SECTIONS] = {};
+    uint64_t row[UKFB_CKPT_SECTIONS] = {}; /* bytes per filter; 0 = one block for all filters (or absent) */
+    uint64_t total = 0;
+};
+
+static CkptLayout ckpt_layout(int kind, long long B, const CkptModes& m)
+{
+    const int LP = kind == UKFB_POSE ? PoseF::LP : OriF::LP, REC = kind == UKFB_POSE ? PoseF::REC : OriF::REC;
+    uint64_t block[UKFB_CKPT_SECTIONS] = {};
+    bool per[UKFB_CKPT_SECTIONS] = {};
+    block[CK_RECORDS] = sizeof(double) * REC, block[CK_T_LAST] = sizeof(int64_t), block[CK_STATUS] = sizeof(uint32_t);
+    block[CK_ACC_MU] = block[CK_GYRO_MU] = sizeof(double) * 3, block[CK_ACC_COV] = sizeof(double) * 9;
+    for (int s = CK_RECORDS; s <= CK_GYRO_MU; ++s) per[s] = true;
+    block[CK_Q] = sizeof(double) * LP, per[CK_Q] = m.q_per_filter != 0;
+    block[CK_ORI] = m.has_ori_params ? sizeof(double) * 5 : 0, per[CK_ORI] = true;
+    for (int k = 0; k < UKFB_MEAS_KIND_COUNT; ++k) {
+        const int d = meas_dim(k);
+        block[CK_MEAS0 + k] = m.meas[k] ? sizeof(double) * d * d : 0;
+        per[CK_MEAS0 + k] = m.meas[k] == 2;
+    }
+    CkptLayout L;
+    uint64_t at = UKFB_CKPT_HEADER_BYTES;
+    for (int s = 0; s < UKFB_CKPT_SECTIONS; ++s) {
+        if (!block[s]) continue;
+        at = align256(at);
+        L.off[s] = at;
+        L.row[s] = per[s] ? block[s] : 0;
+        L.bytes[s] = per[s] ? block[s] * uint64_t(B) : block[s];
+        at += L.bytes[s];
+    }
+    L.total = at;
+    return L;
+}
+
+/* the header of an image of B filters with the handle-wide values of the one-device handle s; hist is left zero */
+static CkptHeader ckpt_header(const ukfb_handle* s, long long B, const CkptModes& m, const CkptLayout& L)
+{
+    CkptHeader hd;
+    memset(&hd, 0, sizeof(hd));
+    memcpy(hd.magic, CKPT_MAGIC, 8);
+    hd.version = UKFB_CHECKPOINT_VERSION, hd.header_bytes = UKFB_CKPT_HEADER_BYTES, hd.total_bytes = L.total;
+    hd.kind = s->kind, hd.MU = s->MU, hd.n = s->n, hd.n_sections = UKFB_CKPT_SECTIONS, hd.B = B;
+    hd.initialized = s->initialized ? 1 : 0, hd.first_init = s->first_init ? 1 : 0;
+    hd.min_dt = s->min_dt, hd.max_dt = s->max_dt, hd.gate_d2 = s->gate_d2;
+    hd.tau_g = s->tau_g, hd.tau_a = s->tau_a, hd.latitude = s->latitude;
+    for (int i = 0; i < 3; ++i) hd.earth[i] = s->earth[i];
+    hd.q_per_filter = m.q_per_filter, hd.has_ori_params = m.has_ori_params;
+    for (int k = 0; k < UKFB_MEAS_KIND_COUNT; ++k) hd.meas_cov_mode[k] = m.meas[k];
+    for (int i = 0; i < UKFB_CKPT_SECTIONS; ++i) hd.section[i] = CkptSection{uint32_t(i), 0u, L.off[i], L.bytes[i]};
+    return hd;
+}
+
+/* every check of a restore, on the host, before anything is enqueued; h: the handle restored into (a parent for a
+ * sharded one).  On success *L is the image's layout. */
+static int ckpt_check(const ukfb_handle* h, const CkptHeader& hd, uint64_t bytes, CkptLayout* L, const char* who)
+{
+    if (memcmp(hd.magic, CKPT_MAGIC, 8) != 0) return fail(UKFB_ERR_INVALID, "%s: not a checkpoint image (bad magic)", who);
+    if (hd.version != UKFB_CHECKPOINT_VERSION || hd.header_bytes != UKFB_CKPT_HEADER_BYTES || hd.n_sections != UKFB_CKPT_SECTIONS)
+        return fail(UKFB_ERR_INVALID, "%s: image version %u (header %u bytes, %u sections); this library reads version %d", who,
+                    hd.version, hd.header_bytes, hd.n_sections, UKFB_CHECKPOINT_VERSION);
+    if (hd.kind != h->kind || hd.B != h->B || hd.MU != h->MU || hd.n != h->n)
+        return fail(UKFB_ERR_INVALID, "%s: the image holds %lld filters of kind %d (MU %d, n %d); this handle %lld of kind %d", who,
+                    (long long)hd.B, hd.kind, hd.MU, hd.n, h->B, h->kind);
+    if (hd.initialized > 1 || hd.first_init > 1 || hd.q_per_filter > 1 || hd.has_ori_params > 1 ||
+        (hd.has_ori_params && h->kind != UKFB_ORIENTATION))
+        return fail(UKFB_ERR_INVALID, "%s: bad flags in the image header", who);
+    CkptModes m;
+    m.q_per_filter = hd.q_per_filter, m.has_ori_params = hd.has_ori_params;
+    for (int k = 0; k < UKFB_MEAS_KIND_COUNT; ++k) {
+        if (hd.meas_cov_mode[k] > 2 || (hd.meas_cov_mode[k] && !kind_ok(h, k)))
+            return fail(UKFB_ERR_INVALID, "%s: bad kept-covariance mode %u for measurement kind %d", who, hd.meas_cov_mode[k], k);
+        m.meas[k] = hd.meas_cov_mode[k];
+    }
+    *L = ckpt_layout(h->kind, h->B, m);
+    for (int s = 0; s < UKFB_CKPT_SECTIONS; ++s) {
+        const CkptSection& e = hd.section[s];
+        if (e.id != uint32_t(s) || e.zero || e.offset != L->off[s] || e.bytes != L->bytes[s])
+            return fail(UKFB_ERR_INVALID, "%s: section %d is %llu bytes at %llu; the header's modes make it %llu bytes at %llu", who, s,
+                        (unsigned long long)e.bytes, (unsigned long long)e.offset, (unsigned long long)L->bytes[s],
+                        (unsigned long long)L->off[s]);
+    }
+    if (hd.total_bytes != L->total || L->total > bytes)
+        return fail(UKFB_ERR_INVALID, "%s: the image needs %llu bytes (header: %llu), %llu given", who, (unsigned long long)L->total,
+                    (unsigned long long)hd.total_bytes, (unsigned long long)bytes);
+    return UKFB_OK;
+}
+
+/* the alignment gaps of an image before each present section: fn(offset, bytes) -- zeroed, so that an image's bytes
+ * depend on the filters' state alone */
+UKFB_HD int ckpt_gaps(const CkptSection* sec, uint64_t at[UKFB_CKPT_SECTIONS], uint64_t len[UKFB_CKPT_SECTIONS])
+{
+    uint64_t end = UKFB_CKPT_HEADER_BYTES;
+    int n = 0;
+    for (int s = 0; s < UKFB_CKPT_SECTIONS; ++s)
+        if (sec[s].bytes) {
+            if (sec[s].offset > end) at[n] = end, len[n++] = sec[s].offset - end;
+            end = sec[s].offset + sec[s].bytes;
+        }
+    return n;
+}
+
+/* the header, its histogram summed over the handle's slots on the device (the header travels as the kernel's argument),
+ * and the zero gaps between sections */
+__global__ void ckpt_header_kernel(const CkptHeader hd, const unsigned long long* __restrict__ hist, unsigned long long* __restrict__ out)
+{
+    const unsigned long long* w = reinterpret_cast<const unsigned long long*>(&hd);
+    for (int i = threadIdx.x; i < UKFB_CKPT_HEADER_BYTES / 8; i += blockDim.x) {
+        const int k = i - int(offsetof(CkptHeader, hist) / 8);
+        unsigned long long v = w[i];
+        if (k >= 0 && k < 8) {
+            v = 0;
+            for (int s = 0; s < HIST_SLOTS; ++s) v += hist[s * 8 + k];
+        }
+        out[i] = v;
+    }
+    char* img = reinterpret_cast<char*>(out);
+    uint64_t at[UKFB_CKPT_SECTIONS], len[UKFB_CKPT_SECTIONS];
+    const int gaps = ckpt_gaps(hd.section, at, len);
+    for (int g = 0; g < gaps; ++g)
+        for (uint64_t j = threadIdx.x; j < len[g]; j += blockDim.x) img[at[g] + j] = 0;
+}
+
+struct CkptHist {
+    unsigned long long w[8];
+};
+/* a restored histogram: all of it in slot 0, the other slots zero */
+__global__ void ckpt_hist_kernel(const CkptHist v, unsigned long long* __restrict__ hist)
+{
+    for (int i = threadIdx.x; i < HIST_SLOTS * 8; i += blockDim.x) hist[i] = i < 8 ? v.w[i] : 0ull;
+}
+
+template <int REC>
+static void ckpt_tile_launch(const ukfb_handle* h, bool save, const CkptParams& p)
+{
+    const long long tiles = (p.B + TILE - 1) / TILE;
+    const unsigned grid = unsigned(std::min<long long>(tiles, 148 * 16));
+    const size_t smem = sizeof(ckpt_word) * ckpt_tile_words(REC); /* one warp per block: 24 / 28 KB, no opt-in needed */
+    if (save)
+        ckpt_save_tile_kernel<REC><<<grid, TILE, smem, h->stream>>>(p);
+    else
+        ckpt_restore_tile_kernel<REC><<<grid, TILE, smem, h->stream>>>(p);
+}
+
+/* records of filters [f0, f0 + n) (f0 a multiple of TILE: whole tiles in either layout start at f0 * REC) <-> n rows.
+ * Per tile through shared memory; UKFB_CKPT_TRANSFORM=elem selects the per-element kernels (DESIGN.md 7.6 compares them) */
+static int ckpt_transform(ukfb_handle* h, bool save, ckpt_word* rows, long long f0, long long n)
+{
+    const CkptParams p{reinterpret_cast<ckpt_word*>(h->state) + f0 * h->REC, rows, n, h->REC, h->tiled};
+    if (knobs().ckpt_elem) {
+        if (save)
+            ckpt_save_elem_kernel<<<grid_for(n * h->REC), 256, 0, h->stream>>>(p);
+        else
+            ckpt_restore_elem_kernel<<<grid_for(n * h->REC), 256, 0, h->stream>>>(p);
+    } else if (h->REC == PoseF::REC)
+        ckpt_tile_launch<PoseF::REC>(h, save, p);
+    else
+        ckpt_tile_launch<OriF::REC>(h, save, p);
+    CU(cudaGetLastError());
+    return UKFB_OK;
+}
+
+/* host-pointer calls move the record section through a device buffer of at most this many bytes, a whole number of tiles
+ * at a time; every other section is dense on the device and goes straight between the caller's buffer and its array */
+constexpr long long CKPT_STAGE_BYTES = 64ll << 20;
+static long long ckpt_chunk(const ukfb_handle* h)
+{
+    const long long per = CKPT_STAGE_BYTES / (long long)(sizeof(double) * h->REC) / TILE * TILE;
+    return std::min<long long>(per, (h->B + TILE - 1) / TILE * TILE);
+}
+
+/* the device arrays behind the sections other than the records, on a one-device handle */
+static void* ckpt_array(ukfb_handle* h, int s)
+{
+    switch (s) {
+        case CK_T_LAST: return h->t_last;
+        case CK_STATUS: return h->status;
+        case CK_ACC_MU: return h->acc_mu;
+        case CK_ACC_COV: return h->acc_cov;
+        case CK_GYRO_MU: return h->gyro_mu;
+        case CK_Q: return h->Q;
+        case CK_ORI: return h->ori_params;
+        default: return h->meas_cov[s - CK_MEAS0];
+    }
+}
+
+/* bytes of section s that a one-device handle of h->B filters holds (its rows of a per-filter section, or the block) */
+static uint64_t ckpt_local_bytes(const ukfb_handle* h, const CkptLayout& G, int s)
+{
+    return G.row[s] ? G.row[s] * uint64_t(h->B) : G.bytes[s];
+}
+
+/* save_dev: the whole image of a one-device handle into d_img, enqueue only */
+static int ckpt_save_enqueue(ukfb_handle* h, char* d_img, const CkptLayout& L, const CkptHeader& hd)
+{
+    ckpt_header_kernel<<<1, 256, 0, h->stream>>>(hd, h->hist, reinterpret_cast<unsigned long long*>(d_img));
+    CU(cudaGetLastError());
+    if (int rc = ckpt_transform(h, true, reinterpret_cast<ckpt_word*>(d_img + L.off[CK_RECORDS]), 0, h->B)) return rc;
+    for (int s = CK_T_LAST; s < UKFB_CKPT_SECTIONS; ++s)
+        if (L.bytes[s]) CU(cudaMemcpyAsync(d_img + L.off[s], ckpt_array(h, s), L.bytes[s], cudaMemcpyDeviceToDevice, h->stream));
+    return UKFB_OK;
+}
+
+/* host save of one device holding filters [first, first + B) of an image of layout G: its rows of every per-filter
+ * section into their places in `buf`, the blocks stored once when first = 0, and its histogram summed into hist[8] */
+static int ckpt_save_part(ukfb_handle* h, long long first, const CkptLayout& G, char* buf, uint64_t hist[8])
+{
+    CHECK_H_AS(h, "ukfb_checkpoint_save"); /* a shard runs this on its worker thread: select its device there */
+    const long long chunk = ckpt_chunk(h);
+    const uint64_t rb = G.row[CK_RECORDS];
+    ckpt_word* d_rows;
+    Staging st(h, false);
+    st.scratch(&d_rows, size_t(chunk * rb));
+    int rc = st.commit();
+    if (rc) return rc;
+    for (long long f0 = 0; f0 < h->B; f0 += chunk) { /* the next chunk's transform waits for this chunk's copy: one stream */
+        const long long n = std::min(chunk, h->B - f0);
+        if ((rc = ckpt_transform(h, true, d_rows, f0, n))) return rc;
+        CU(cudaMemcpyAsync(buf + G.off[CK_RECORDS] + uint64_t(first + f0) * rb, d_rows, size_t(n * rb), cudaMemcpyDeviceToHost, h->stream));
+    }
+    for (int s = CK_T_LAST; s < UKFB_CKPT_SECTIONS; ++s)
+        if (G.bytes[s] && (G.row[s] || first == 0))
+            CU(cudaMemcpyAsync(buf + G.off[s] + uint64_t(first) * G.row[s], ckpt_array(h, s), ckpt_local_bytes(h, G, s), cudaMemcpyDeviceToHost,
+                               h->stream));
+    unsigned long long slots[HIST_SLOTS * 8];
+    CU(cudaMemcpyAsync(slots, h->hist, sizeof(slots), cudaMemcpyDeviceToHost, h->stream));
+    if ((rc = st.finish())) return rc;
+    for (int k = 0; k < 8; ++k) {
+        hist[k] = 0;
+        for (int j = 0; j < HIST_SLOTS; ++j) hist[k] += slots[j * 8 + k];
+    }
+    return UKFB_OK;
+}
+
+/* restore of one device holding filters [first, first + B) from an image of layout G with the checked header hd:
+ * src is the image in host memory (host-pointer call: records staged by chunks, blocking) or in this device's memory
+ * (restore_dev: enqueue only).  hist_here: the image's histogram goes to this device, else its histogram is cleared.
+ * q_host: the image's broadcast Q (LP doubles, host), or null when per filter.  Buffers whose mode changes are all
+ * allocated before any old one is freed, so a failed allocation leaves this device's handle as it was. */
+static int ckpt_restore_part(ukfb_handle* h, long long first, const CkptLayout& G, const char* src, bool src_dev, const CkptHeader& hd,
+                             bool hist_here, const double* q_host, const char* who)
+{
+    CHECK_H_AS(h, who);
+    const long long chunk = ckpt_chunk(h);
+    const uint64_t rb = G.row[CK_RECORDS];
+    ckpt_word* d_rows = nullptr;
+    Staging st(h, false);
+    if (!src_dev) {
+        st.scratch(&d_rows, size_t(chunk * rb));
+        if (int rc = st.commit()) return rc;
+    }
+    /* the arrays whose size changes with the image's modes: new ones first */
+    double** slot[2 + UKFB_MEAS_KIND_COUNT];
+    double* fresh[2 + UKFB_MEAS_KIND_COUNT];
+    int sec[2 + UKFB_MEAS_KIND_COUNT], nr = 0;
+    if (int(hd.q_per_filter) != h->q_per_filter) slot[nr] = &h->Q, sec[nr++] = CK_Q;
+    if (bool(hd.has_ori_params) != (h->ori_params != nullptr)) slot[nr] = &h->ori_params, sec[nr++] = CK_ORI;
+    for (int k = 0; k < UKFB_MEAS_KIND_COUNT; ++k)
+        if (int(hd.meas_cov_mode[k]) != h->meas_cov_per_filter[k]) slot[nr] = &h->meas_cov[k], sec[nr++] = CK_MEAS0 + k;
+    for (int i = 0; i < nr; ++i) {
+        fresh[i] = nullptr;
+        const uint64_t bytes = ckpt_local_bytes(h, G, sec[i]);
+        const cudaError_t e = bytes ? cudaMalloc(&fresh[i], bytes) : cudaSuccess;
+        if (e != cudaSuccess) {
+            for (int j = 0; j < i; ++j) cudaFree(fresh[j]);
+            return fail(UKFB_ERR_NOMEM, "%s: %s", who, cudaGetErrorString(e));
+        }
+    }
+    if (nr) {
+        CU(cudaStreamSynchronize(h->stream)); /* nothing may still read the old arrays */
+        for (int i = 0; i < nr; ++i) {
+            cudaFree(*slot[i]);
+            *slot[i] = fresh[i];
+        }
+    }
+    h->q_per_filter = int(hd.q_per_filter);
+    for (int k = 0; k < UKFB_MEAS_KIND_COUNT; ++k) h->meas_cov_per_filter[k] = int(hd.meas_cov_mode[k]);
+    const cudaMemcpyKind kind = src_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    int rc = UKFB_OK;
+    if (src_dev)
+        rc = ckpt_transform(h, false, reinterpret_cast<ckpt_word*>(const_cast<char*>(src) + G.off[CK_RECORDS]), 0, h->B);
+    else
+        for (long long f0 = 0; f0 < h->B && !rc; f0 += chunk) { /* this chunk's copy waits for the last chunk's transform */
+            const long long n = std::min(chunk, h->B - f0);
+            CU(cudaMemcpyAsync(d_rows, src + G.off[CK_RECORDS] + uint64_t(first + f0) * rb, size_t(n * rb), cudaMemcpyHostToDevice, h->stream));
+            rc = ckpt_transform(h, false, d_rows, f0, n);
+        }
+    if (rc) return rc;
+    for (int s = CK_T_LAST; s < UKFB_CKPT_SECTIONS; ++s)
+        if (G.bytes[s]) CU(cudaMemcpyAsync(ckpt_array(h, s), src + G.off[s] + uint64_t(first) * G.row[s], ckpt_local_bytes(h, G, s), kind, h->stream));
+    CkptHist hv;
+    for (int k = 0; k < 8; ++k) hv.w[k] = hist_here ? hd.hist[k] : 0ull;
+    ckpt_hist_kernel<<<1, 256, 0, h->stream>>>(hv, h->hist);
+    CU(cudaGetLastError());
+    h->q_diagonal = hd.q_per_filter ? 0 : broadcast_q_class(q_host, h->n);
+    h->min_dt = hd.min_dt, h->max_dt = hd.max_dt, h->gate_d2 = hd.gate_d2;
+    h->tau_g = hd.tau_g, h->tau_a = hd.tau_a, h->latitude = hd.latitude;
+    for (int i = 0; i < 3; ++i) h->earth[i] = hd.earth[i];
+    h->initialized = hd.initialized != 0, h->first_init = hd.first_init != 0;
+    return src_dev ? UKFB_OK : st.finish();
+}
+
+/* restore_dev's one read-back: the header and, where the header's Q section is one block that lies inside the image,
+ * that block behind it (checked on the host afterwards like every other field) */
+__global__ void ckpt_probe_kernel(const unsigned char* __restrict__ img, uint64_t bytes, unsigned char* __restrict__ out)
+{
+    const CkptSection* q = reinterpret_cast<const CkptSection*>(img + offsetof(CkptHeader, section)) + CK_Q;
+    for (int i = threadIdx.x; i < UKFB_CKPT_HEADER_BYTES; i += blockDim.x) out[i] = img[i];
+    const uint64_t off = q->offset, n = q->bytes;
+    if (n && n <= sizeof(double) * OriF::LP && off >= UKFB_CKPT_HEADER_BYTES && off <= bytes && n <= bytes - off)
+        for (uint64_t i = threadIdx.x; i < n; i += blockDim.x) out[UKFB_CKPT_HEADER_BYTES + i] = img[off + i];
+}
+
+extern "C" int ukfb_checkpoint_size(ukfb_handle* h, uint64_t* bytes)
+{
+    if (!h || !bytes) return fail(UKFB_ERR_INVALID, "ukfb_checkpoint_size: null argument");
+    *bytes = ckpt_layout(h->kind, h->B, ckpt_modes(h)).total;
+    return UKFB_OK;
+}
+
+extern "C" int ukfb_checkpoint_save(ukfb_handle* h, void* buf, uint64_t bytes)
+{
+    CHECK_H(h);
+    NEED_INIT(h);
+    const CkptModes m = ckpt_modes(h);
+    const CkptLayout G = ckpt_layout(h->kind, h->B, m);
+    if (!buf) return fail(UKFB_ERR_INVALID, "ukfb_checkpoint_save: null buffer");
+    if (bytes < G.total)
+        return fail(UKFB_ERR_INVALID, "ukfb_checkpoint_save: the image needs %llu bytes, the buffer has %llu", (unsigned long long)G.total,
+                    (unsigned long long)bytes);
+    char* out = static_cast<char*>(buf);
+    CkptHeader hd = ckpt_header(is_sharded(h) ? h->shards[0] : h, h->B, m, G);
+    uint64_t at[UKFB_CKPT_SECTIONS], len[UKFB_CKPT_SECTIONS];
+    for (int g = ckpt_gaps(hd.section, at, len) - 1; g >= 0; --g) memset(out + at[g], 0, len[g]); /* the sections go in concurrently */
+    std::vector<std::array<uint64_t, 8>> part(h->shards.empty() ? 1 : h->shards.size());
+    const int rc = is_sharded(h) ? fan_out(h, [&](ukfb_handle* s_, long long f_, long long) { return ckpt_save_part(s_, f_, G, out, part[shard_at(h, f_)].data()); })
+                                 : ckpt_save_part(h, 0, G, out, part[0].data());
+    if (rc) return rc;
+    /* handle-wide values of shard 0 (every setter fans out: the shards agree), the histogram summed over the shards */
+    for (const auto& p : part)
+        for (int k = 0; k < 8; ++k) hd.hist[k] += p[size_t(k)];
+    memcpy(out, &hd, sizeof(hd));
+    return UKFB_OK;
+}
+
+extern "C" int ukfb_checkpoint_restore(ukfb_handle* h, const void* buf, uint64_t bytes)
+{
+    CHECK_H(h);
+    if (!buf) return fail(UKFB_ERR_INVALID, "ukfb_checkpoint_restore: null buffer");
+    if (bytes < sizeof(CkptHeader))
+        return fail(UKFB_ERR_INVALID, "ukfb_checkpoint_restore: %llu bytes cannot hold an image", (unsigned long long)bytes);
+    const char* in = static_cast<const char*>(buf);
+    CkptHeader hd;
+    memcpy(&hd, in, sizeof(hd));
+    CkptLayout G;
+    int rc = ckpt_check(h, hd, bytes, &G, "ukfb_checkpoint_restore");
+    if (rc) return rc;
+    double q[OriF::LP]; /* the broadcast Q, copied out: the caller's buffer need not be aligned */
+    if (!hd.q_per_filter) memcpy(q, in + G.off[CK_Q], G.bytes[CK_Q]);
+    const double* qp = hd.q_per_filter ? nullptr : q;
+    if (!is_sharded(h)) return ckpt_restore_part(h, 0, G, in, false, hd, true, qp, "ukfb_checkpoint_restore");
+    /* a shard that cannot allocate fails alone: the others are restored (UKFB_ERR_NOMEM names the shard) */
+    rc = fan_out(h, [&](ukfb_handle* s_, long long f_, long long) { return ckpt_restore_part(s_, f_, G, in, false, hd, f_ == 0, qp, "ukfb_checkpoint_restore"); });
+    if (rc) return rc;
+    /* the parent's own copies of handle-wide values (the setters keep them too) */
+    h->min_dt = hd.min_dt, h->max_dt = hd.max_dt, h->gate_d2 = hd.gate_d2;
+    h->tau_g = hd.tau_g, h->tau_a = hd.tau_a, h->latitude = hd.latitude;
+    for (int i = 0; i < 3; ++i) h->earth[i] = hd.earth[i];
+    for (int k = 0; k < UKFB_MEAS_KIND_COUNT; ++k) h->meas_cov_per_filter[k] = int(hd.meas_cov_mode[k]);
+    h->initialized = hd.initialized != 0, h->first_init = hd.first_init != 0;
+    return UKFB_OK;
+}
+
+extern "C" int ukfb_checkpoint_save_dev(ukfb_handle* h, void* d_buf, uint64_t bytes)
+{
+    CHECK_H(h);
+    UKFB_NOT_SHARDED(h);
+    NEED_INIT(h);
+    const CkptModes m = ckpt_modes(h);
+    const CkptLayout L = ckpt_layout(h->kind, h->B, m);
+    if (!d_buf) return fail(UKFB_ERR_INVALID, "ukfb_checkpoint_save_dev: null buffer");
+    if (bytes < L.total)
+        return fail(UKFB_ERR_INVALID, "ukfb_checkpoint_save_dev: the image needs %llu bytes, the buffer has %llu",
+                    (unsigned long long)L.total, (unsigned long long)bytes);
+    return ckpt_save_enqueue(h, static_cast<char*>(d_buf), L, ckpt_header(h, h->B, m, L));
+}
+
+extern "C" int ukfb_checkpoint_restore_dev(ukfb_handle* h, const void* d_buf, uint64_t bytes)
+{
+    CHECK_H(h);
+    UKFB_NOT_SHARDED(h);
+    if (!d_buf) return fail(UKFB_ERR_INVALID, "ukfb_checkpoint_restore_dev: null buffer");
+    if (bytes < sizeof(CkptHeader))
+        return fail(UKFB_ERR_INVALID, "ukfb_checkpoint_restore_dev: %llu bytes cannot hold an image", (unsigned long long)bytes);
+    const char* in = static_cast<const char*>(d_buf);
+    const size_t probe = UKFB_CKPT_HEADER_BYTES + sizeof(double) * OriF::LP;
+    int rc = stage_grow(h, h->stage, h->stage_bytes, probe, false);
+    if (rc) return rc;
+    ckpt_probe_kernel<<<1, 256, 0, h->stream>>>(reinterpret_cast<const unsigned char*>(in), bytes, reinterpret_cast<unsigned char*>(h->stage));
+    CU(cudaGetLastError());
+    unsigned char back[UKFB_CKPT_HEADER_BYTES + sizeof(double) * OriF::LP];
+    CU(cudaMemcpyAsync(back, h->stage, probe, cudaMemcpyDeviceToHost, h->stream)); /* after whatever wrote the image on this stream */
+    CU(cudaStreamSynchronize(h->stream));
+    CkptHeader hd;
+    memcpy(&hd, back, sizeof(hd));
+    CkptLayout L;
+    rc = ckpt_check(h, hd, bytes, &L, "ukfb_checkpoint_restore_dev");
+    if (rc) return rc;
+    double q[OriF::LP]; /* checked: a broadcast Q section is one block inside the image, so the probe copied it */
+    if (!hd.q_per_filter) memcpy(q, back + UKFB_CKPT_HEADER_BYTES, L.bytes[CK_Q]);
+    return ckpt_restore_part(h, 0, L, in, true, hd, true, hd.q_per_filter ? nullptr : q, "ukfb_checkpoint_restore_dev");
 }
 
 /* ---- stream plumbing ------------------------------------------------------------------------------------------ */

@@ -9,7 +9,7 @@ UKFB_EMU_SANITIZE=1 LD_PRELOAD="$ASAN $STDCPP" \
   ASAN_OPTIONS=detect_leaks=0:halt_on_error=1:log_path=/tmp/ukfb_asan \
   UBSAN_OPTIONS=halt_on_error=1:print_stacktrace=1:log_path=/tmp/ukfb_ubsan \
   python -m pytest tests/test_emu_lane_kernels.py tests/test_emu_parity.py tests/test_gate.py tests/test_events.py \
-    tests/test_so3_kernels.py tests/test_emu_indexed.py -x -q -m "not gpu" -p no:cacheprovider
+    tests/test_so3_kernels.py tests/test_emu_indexed.py tests/test_emu_checkpoint.py -x -q -m "not gpu" -p no:cacheprovider
 rc=$?
 ls /tmp/ukfb_asan.* /tmp/ukfb_ubsan.* 2>/dev/null && { echo "sanitizer reports written"; rc=1; }
 exit $rc
