@@ -22,12 +22,23 @@ using namespace orc;
 /* The filter objects behind the batch.  Default: the oracle's own restatement of the reference classes.  oracle/ref_capi.cpp
  * defines ORC_CUSTOM_IMPL, adapters over the REFERENCE'S OWN classes (compiled unmodified from /root/reference against
  * oracle/ref_shim) with the same member functions, and includes this file: the same batch interface then drives them. */
+/* ORC_REAL: the filters' scalar.  `double` is the oracle proper; liboracle_ld.so builds with `long double` as an
+ * extended-precision reference for the FP64 implementations.  The C interface stays `double` either way: inputs
+ * widen exactly and results are rounded once on read-back. */
+#ifndef ORC_REAL
+#define ORC_REAL double
+#endif
+
 #ifndef ORC_CUSTOM_IMPL
-typedef PoseFilter<double> PoseImpl;
-typedef OrientationFilter<double> OriImpl;
+typedef PoseFilter<ORC_REAL> PoseImpl;
+typedef OrientationFilter<ORC_REAL> OriImpl;
 namespace ax { /* access to what the reference keeps in protected members / inside ukfom::ukf */
 template <class F> void store_mu(const F& f, double* mu) { f.ukf.mu.store(mu); }
-template <class F> void copy_sigma(const F& f, double* sigma) { std::memcpy(sigma, f.ukf.sigma, sizeof(f.ukf.sigma)); }
+template <class F> void copy_sigma(const F& f, double* sigma)
+{
+    const int nn = sizeof(f.ukf.sigma) / sizeof(f.ukf.sigma[0]);
+    for (int k = 0; k < nn; ++k) sigma[k] = double(f.ukf.sigma[k]);
+}
 template <class F> void set_q(F& f, int k, double v) { f.process_noise_cov[k] = v; }
 template <class F> void set_dt_bounds(F& f, double lo, double hi) { f.min_time_delta = lo, f.max_time_delta = hi; }
 template <class F> void set_gate(F& f, double d2) { f.ukf.accept_max_d2 = d2; }
@@ -133,22 +144,24 @@ int orc_initialize(void* h, const double* mu, const double* sigma)
     }
 #pragma omp parallel for schedule(static)
     for (int64_t i = 0; i < b->B; ++i) {
+        ORC_REAL sg[UKFB_ORI_DOF * UKFB_ORI_DOF]; /* the larger of the two kinds */
+        for (int k = 0; k < nn; ++k) sg[k] = sigma[i * nn + k];
         if (b->kind == 0) {
-            PoseState<double> s;
+            PoseState<ORC_REAL> s;
             s.load(mu + i * b->MU);
             if (!b->constructed) {
-                b->pose[i].reset(new PoseImpl(s, sigma + i * nn));
+                b->pose[i].reset(new PoseImpl(s, sg));
                 apply_common(b, *b->pose[i], i);
             } else
-                b->pose[i]->initializeFilter(s, sigma + i * nn);
+                b->pose[i]->initializeFilter(s, sg);
         } else {
-            OrientationState<double> s;
+            OrientationState<ORC_REAL> s;
             s.load(mu + i * b->MU);
             if (!b->constructed) {
-                b->ori[i].reset(new OriImpl(s, sigma + i * nn, b->tau_g, b->tau_a, b->latitude));
+                b->ori[i].reset(new OriImpl(s, sg, b->tau_g, b->tau_a, b->latitude));
                 apply_common(b, *b->ori[i], i);
             } else
-                b->ori[i]->initializeFilter(s, sigma + i * nn);
+                b->ori[i]->initializeFilter(s, sg);
         }
     }
     b->constructed = true;

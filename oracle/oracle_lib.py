@@ -38,8 +38,9 @@ def build_ref(quiet: bool = True) -> bool:
 
 
 def load(variant: str = "left") -> C.CDLL:
-    """variant: 'left' (default SO(3) convention), 'right' (upstream body-frame) or 'ref' (the reference's own wrapper
-    sources over the oracle's engine, oracle/_ref)."""
+    """variant: 'left' (default SO(3) convention), 'right' (upstream body-frame), 'tight' (tighter manifold-mean
+    tolerance), 'ld' (the default oracle computed in long double, tests/precision.py) or 'ref' (the reference's own
+    wrapper sources over the oracle's engine, oracle/_ref)."""
     if variant in _LIBS:
         return _LIBS[variant]
     if variant == "ref":
@@ -47,7 +48,8 @@ def load(variant: str = "left") -> C.CDLL:
             raise RuntimeError("oracle/_ref/libref.so is missing and /root/reference is not here to build it")
         path = REF_LIB
     else:
-        name = {"left": "liboracle.so", "right": "liboracle_right.so", "tight": "liboracle_tight.so"}[variant]
+        name = {"left": "liboracle.so", "right": "liboracle_right.so", "tight": "liboracle_tight.so",
+                "ld": "liboracle_ld.so"}[variant]
         path = os.path.join(_DIR, "build", name)
         if not os.path.exists(path):
             build()

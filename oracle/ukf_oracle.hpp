@@ -25,9 +25,12 @@
  * (slam_pose_estimation_b200/) never does.
  *
  * Everything is a template over the scalar T so that the same code runs with
- * `double` (the oracle proper) and with a counting scalar (oracle/count_ops.cpp)
- * that measures the algorithmic flop / special-function counts of SURVEY.md
- * section 8(d).
+ * `double` (the oracle proper), with `long double` (liboracle_ld.so, the
+ * extended-precision reference of tests/precision.py) and with a counting scalar
+ * (oracle/count_ops.cpp) that measures the algorithmic flop / special-function
+ * counts of SURVEY.md section 8(d).  Only inputs stay `double` (dt, z, R, the
+ * stored IMU / acceleration samples, tau, the earth rate): every intermediate of
+ * Ukf<T,S>, the models and rotate_block is a T.
  *
  * Each function cites the reference file:line (or the upstream MTK file) it follows.
  */
@@ -63,6 +66,20 @@ enum : uint32_t {
 
 template <class T>
 inline bool is_finite(const T& x) { return std::isfinite(static_cast<double>(x)); }
+
+/* a floating-point scalar wider than double (the extended-precision reference) */
+template <class T>
+constexpr bool kWiderThanDouble = std::is_floating_point<T>::value && (sizeof(T) > sizeof(double));
+
+/* 1/k: the double constant for double and for the counting scalar, rounded in T itself when T is wider */
+template <class T>
+inline T recip(int k)
+{
+    if constexpr (kWiderThanDouble<T>)
+        return T(1) / T(k);
+    else
+        return T(1. / k);
+}
 
 /* ------------------------------------------------------------------------- */
 /* Quaternion, Eigen::Quaternion<double> semantics, storage (x,y,z,w).         */
@@ -150,14 +167,13 @@ inline void cos_sinc_sqrt(const T& x2, T& c, T& sinc)
         sinc = sin(x) / x;
         return;
     }
-    static const double inv[] = {1 / 3., 1 / 4., 1 / 5., 1 / 6., 1 / 7., 1 / 8., 1 / 9.};
     T cosi = T(1), si = T(1);
     T term = T(-1 / 2.) * x2;
     for (int i = 0; i < 3; ++i) {
         cosi = cosi + term;
-        term = term * T(inv[2 * i]);
+        term = term * recip<T>(2 * i + 3);
         si = si + term;
-        term = term * (T(-inv[2 * i + 1]) * x2);
+        term = term * (-recip<T>(2 * i + 4) * x2);
     }
     c = cosi;
     sinc = si;
@@ -943,7 +959,7 @@ public:
         T er[3] = {T(earth_rotation[0]), T(earth_rotation[1]), T(earth_rotation[2])};
         T r[3];
         quat_rotate(quat_inverse(this->ukf.mu.orientation), er, r);
-        for (int i = 0; i < 3; ++i) out[i] = rotation_rate_mu[i] - double(this->ukf.mu.bias_gyro[i]) - double(r[i]);
+        for (int i = 0; i < 3; ++i) out[i] = double(T(rotation_rate_mu[i]) - this->ukf.mu.bias_gyro[i] - r[i]);
     }
 
     /* :12-32 -- the acceleration is rotated with the UPDATED orientation. */
@@ -988,7 +1004,12 @@ protected:
         for (int i = 0; i < n * n; ++i) process_noise[i] = this->process_noise_cov[i];
         Base::rotate_block(process_noise, this->process_noise_cov, rot, 0);
         Base::rotate_block(process_noise, this->process_noise_cov, rot, 3);
-        const T d2 = T(std::pow(delta, 2.));
+        /* a scalar wider than double squares the exact delta; double keeps the reference's std::pow */
+        T d2;
+        if constexpr (kWiderThanDouble<T>)
+            d2 = T(delta) * T(delta);
+        else
+            d2 = T(std::pow(delta, 2.));
         for (int i = 0; i < n * n; ++i) process_noise[i] = d2 * process_noise[i];
 
         const T a[3] = {T(acceleration_mu[0]), T(acceleration_mu[1]), T(acceleration_mu[2])};
